@@ -3,10 +3,16 @@
 
 Contract: `python bench.py --gpus N --steps K --warmup W` (N>1: launched by torch.distributed.run) prints ONE
 JSON line on rank 0.  A "step" is one compute() pass of the hot path over one batch of synthetic paths.
+`--steps K` sets the timed steps of the headline and of the em sub-record; the other sub-records time fixed counts (below).
 
 Headline (the line's own metric/value): BASELINE.json configs[1] -- FE Euler, N=1000 time steps, 2^24 paths per GPU,
 README parameters, seed 1234.  Paths shard over ranks by disjoint Philox subsequences (weak scaling); one NCCL
 allreduce of the two FP64 moments per step when N>1.
+
+`--dump-outputs DIR` writes what each timed path returned in its last timed step, the FP64 sums (payoff, payoff^2), as
+DIR/<name>.npy: `moments` (headline), and with the sub-records `em_moments`, `c5_fe_moments`, `c5_em_moments` and
+`c4_fe_moments` / `c4_em_moments` (one row per grid point).  Seeds are fixed, so the same arguments give the same inputs
+and two builds can be compared output for output.
 
   value     FE: path-steps/s, whole job; inputs are 11 scalars (nothing to stage in HBM)
   e2e       the same metric through the public C-ABI call nmch_engine_compute() with host buffers:
@@ -57,6 +63,7 @@ EM_TRIALS_PER_STEP = 1.045                                # Marsaglia-Tsang acce
 # SURVEY.md §8d for EM: "estimate 90-100 instr/step => 3.9e8 paths/s/GPU ceiling at N=1000" = 95 thread-instr per
 # path-step at one instruction per scheduler per clock
 EM_INSTR_PER_PATH_STEP = 95.0
+DUMP_LIMIT_BYTES = 64 << 20                               # --dump-outputs writes at most this much in all
 
 
 # ------------------------------------------------------------------------------------------------
@@ -287,7 +294,9 @@ def reference_cuda_plus_floor(n: int, N: int, repeat: int = 3):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline and of the em sub-record; c5_strong times a fixed 3 (2^30 paths per "
+                         "step), c4_sweep one launch, other_floor / dense_mode / xorwow_fast_mode the best of 3")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--method", default="fe", choices=["fe", "em"])
@@ -305,7 +314,16 @@ def main():
     ap.add_argument("--c4-log2-paths", type=int, default=20, help="GLOBAL paths per grid point of the c4_sweep sub-record")
     ap.add_argument("--c4-points", type=int, default=20, help="grid points per axis of the c4_sweep sub-record")
     ap.add_argument("--cpu-budget-s", type=float, default=None, help="seconds of host work per CPU-baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each timed path returned in its last timed step as DIR/<name>.npy (FP64 moment sums)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU paths' results: it needs --impl ours")
+    # the c4 arrays (16 bytes per grid point and method, at most c4_points^3 points) are the only ones that grow
+    if args.dump_outputs and not args.no_sub_records and 2 * 16 * args.c4_points ** 3 > DUMP_LIMIT_BYTES - 1024:
+        ap.error(f"--dump-outputs: --c4-points {args.c4_points} would write more than {DUMP_LIMIT_BYTES >> 20} MB")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -378,6 +396,9 @@ def main():
     from nmch_b200.distributed import ShardedEngine
     stream = torch.cuda.Stream(dev)             # one stream carries the kernel and the allreduce
     torch.cuda.set_stream(stream)
+
+    # name -> what a timed path returned in its last timed step (FP64 moment sums), for --dump-outputs
+    outputs = {}
 
     def barrier():
         if world > 1:
@@ -468,6 +489,7 @@ def main():
         launches = sh.engine.launch_info()["kernel_launches"] - l0
         sums = buf.cpu().numpy().reshape(-1, 2)
         sh.close()
+        outputs[f"c4_{method}_moments"] = sums
         means = sums[:, 0] / n_global
         units = len(k_) * n_global * (N if method == "fe" else 1)
         i0 = int(np.argmin(np.abs(k_ - 0.5) + np.abs(t_ - 0.1) * 10 + np.abs(s_ - 0.3) * 3))
@@ -517,17 +539,19 @@ def main():
     head_rng = E.RNG_PHILOX_DENSE if (args.rng == "dense" and args.method == "fe") else E.RNG_PHILOX
     head = measure(args.method, n_per_gpu * world, args.steps, args.warmup, rng=head_rng, sample_clocks=True)
     assert head["n_local"] == n_per_gpu
+    outputs["moments"] = head["result"]
 
     # ---- sub-records (every N): the EM half of BASELINE.json's metric, and configs[4] as strong scaling
     sub = {}
     if not args.no_sub_records and args.method == "fe" and args.rng == "philox":
-        em_steps = max(3, min(args.steps, 10))
-        em = measure("em", (1 << 22) * world, em_steps, 3, sample_clocks=True)
+        em = measure("em", (1 << 22) * world, args.steps, 3, sample_clocks=True)
         sub["em"] = em
+        outputs["em_moments"] = em["result"]
         c5_n = 1 << args.c5_log2_paths
         c5 = {}
         for m in ("fe", "em"):
             c5[m] = measure(m, c5_n, 3, 1, want_e2e=False)
+            outputs[f"c5_{m}_moments"] = c5[m]["result"]
         sub["c5"] = (c5_n, c5)
         sub["c4"] = {m: sweep(m, 1 << args.c4_log2_paths, args.c4_points) for m in ("fe", "em")}
 
@@ -587,7 +611,7 @@ def main():
             eck = em["clocks"]
             line["em"] = {
                 "metric": "em_paths_per_s", "value": em["value"], "unit": "paths/s", "ms_per_step": em["ms_per_step"],
-                "steps": max(3, min(args.steps, 10)), "warmup": 3, "scaling": "weak", "gpu_launches": em["launches"],
+                "steps": args.steps, "warmup": 3, "scaling": "weak", "gpu_launches": em["launches"],
                 "config": {"workload": f"BASELINE configs[2]: EM exact scheme, README params, N={N}, 2^22 paths per GPU, seed 1234",
                            "paths_per_gpu": 1 << 22, "global_paths": (1 << 22) * world},
                 "e2e": em["e2e"], "clocks": eck,
@@ -663,6 +687,11 @@ def main():
             line["reference_cuda"] = reference_cuda(args.method, log2_paths, N)
             if "em" in line:
                 line["em"]["reference_cuda"] = reference_cuda("em", 22, N, spread_runs=2)
+        if args.dump_outputs:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), np.asarray(arr, dtype=np.float64))
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

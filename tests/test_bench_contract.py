@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,17 +32,38 @@ def test_reference_arm_line():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_dump_outputs_over_64_mb_is_refused():
+    """--dump-outputs writes at most 64 MB: a grid whose c4 arrays would exceed that is rejected before any work."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", "unused", "--c4-points", "130"],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 2 and "more than 64 MB" in r.stderr, r.stderr[-400:]
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("method,metric", [("fe", "fe_path_steps_per_s"), ("em", "em_paths_per_s")])
-def test_our_arm_line(method, metric):
+@pytest.mark.parametrize("method,metric",[("fe", "fe_path_steps_per_s"), ("em", "em_paths_per_s")])
+def test_our_arm_line(method, metric, tmp_path):
     d = _run("--method", method, "--steps", "3", "--warmup", "3", "--log2-paths", "20", "--cpu-budget-s", "0.3", "--no-reference-cuda",
-             "--no-sub-records")
+             "--no-sub-records", "--dump-outputs", str(tmp_path))
     assert BASE_KEYS | {"gpu_launches", "clocks", "roofline", "kernel"} <= set(d)
     assert d["metric"] == metric and d["n_gpus"] == 1 and d["gpu_launches"] == 3 and d["value"] > 0
     assert set(d["roofline"]) >= {"bound", "achieved", "peak", "unit", "frac", "traffic"}
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     assert d["e2e"]["h2d_bytes_per_step"] > 0 and d["e2e"]["d2h_bytes_per_step"] == 16
     assert abs(d["result"]["E[X]"] - 0.1197325) < 5 * d["result"]["std_error"] + 2e-4
+    # --dump-outputs: the FP64 sums of the last timed step, the ones the line's result is derived from
+    assert sorted(os.listdir(tmp_path)) == ["moments.npy"]
+    m = np.load(tmp_path / "moments.npy")
+    assert m.dtype == np.float64 and m.shape == (2,)
+    assert m[0] / (1 << 20) == d["result"]["E[X]"]
+    # ... and they are call warmup + steps = 6 of the seeded stream, not a warm-up step or an earlier one
+    from nmch_b200 import engine as E
+    with E.Engine(NTPB=512, NB=(1 << 20) // 512, N=1000, method=E.METHOD_FE if method == "fe" else E.METHOD_EM,
+                  rng=E.RNG_PHILOX) as e:
+        e.init(1234)
+        calls = [e.compute() for _ in range(6)]
+    last, before = np.array([calls[5].sum_payoff, calls[5].sum_payoff_sq]), np.array([calls[4].sum_payoff, calls[4].sum_payoff_sq])
+    np.testing.assert_allclose(m, last, rtol=1e-12)
+    assert np.abs(m - before).max() > 1e-6 * np.abs(before).max()
 
 
 def test_reference_arm_uses_every_host_thread_under_torchrun_env():
@@ -62,9 +84,9 @@ def test_reference_arm_uses_every_host_thread_under_torchrun_env():
 
 
 @pytest.mark.gpu
-def test_sub_records_em_and_c5_strong():
+def test_sub_records_em_and_c5_strong(tmp_path):
     d = _run("--steps", "3", "--warmup", "3", "--log2-paths", "20", "--c5-log2-paths", "22", "--c4-log2-paths", "14", "--c4-points", "6",
-             "--no-cpu-baseline", "--no-reference-cuda")
+             "--no-cpu-baseline", "--no-reference-cuda", "--dump-outputs", str(tmp_path))
     assert d["metric"] == "fe_path_steps_per_s" and d["gpu_launches"] == 3
     em = d["em"]
     assert em["metric"] == "em_paths_per_s" and em["unit"] == "paths/s" and em["value"] > 0 and em["gpu_launches"] == em["steps"]
@@ -81,6 +103,11 @@ def test_sub_records_em_and_c5_strong():
     c4 = d["c4_sweep"]
     for m in ("fe", "em"):
         assert c4[m]["gpu_launches"] == 1 and c4[m]["all_finite"] and c4[m]["points"] == 200 and c4[m]["launch_ms"] > 0
+    # --dump-outputs: one file per timed path
+    assert sorted(os.listdir(tmp_path)) == sorted(f"{n}.npy" for n in ("moments", "em_moments", "c5_fe_moments", "c5_em_moments",
+                                                                          "c4_fe_moments", "c4_em_moments"))
+    assert np.load(tmp_path / "em_moments.npy")[0] / (1 << 22) == em["result"]["E[X]"]
+    assert np.load(tmp_path / "c4_fe_moments.npy").shape == (200, 2)
 
 
 @pytest.mark.gpu

@@ -68,12 +68,10 @@ def test_nmch_report_matches_reference_format(method, title):
 
 @pytest.mark.gpu
 def test_nmch_xorwow_tag_matches_reference_binary():
-    from oracle import oracle as o
-    if not os.path.exists(o.REF_HARNESS_PATH):
-        pytest.skip("reference harness not shipped")
+    from ref_build import harness_rows
     r = run(NMCH, "--rng", "xorwow", "--NB", 128, "--N", 300, "--json")
     j = json.loads(r.stdout.splitlines()[-1])
-    ref = json.loads(run(o.REF_HARNESS_PATH, "--method", "fe", "--rng", "xorwow", "--NB", 128, "--N", 300).stdout.splitlines()[0])
+    ref = harness_rows(method="fe", rng="xorwow", NB=128, N=300)[0]
     assert abs(j["E"] - ref["E"]) / ref["E"] < 1e-5
     assert abs(j["err"] - ref["err"]) / ref["err"] < 1e-4          # the reference's own CI formula, same inputs
 

@@ -171,15 +171,10 @@ def test_every_class_name_matches_the_same_class_of_the_reference_build(matrix_e
     compared statistically elsewhere (tests/test_gpu_em.py).  K1-family classes with set_legacy_k1_moment(true): their
     price_squared is the reference's E[X^2]/n^2 (NMCH_FE.cu:56-58)."""
     import json
-    from oracle import oracle as o
-    if not os.path.exists(o.REF_HARNESS_PATH):
-        pytest.skip("oracle/_ref/nmch_ref_harness not shipped")
+    from ref_build import harness_rows
     NTPB, NB, N = (256, 64, 120) if method == "fe" else (128, 32, 60)      # K1 needs a power-of-two block (NMCH_FE.cu:62-72)
     for tag in tags:
-        ref = subprocess.run([o.REF_HARNESS_PATH, "--method", method, "--rng", tag, "--kernel", kernel, "--NTPB", str(NTPB),
-                              "--NB", str(NB), "--N", str(N), "--repeat", "2"], capture_output=True, text=True, timeout=600)
-        assert ref.returncode == 0, ref.stderr[-400:]
-        want = [json.loads(l.replace("-nan", "NaN").replace(" nan", " NaN")) for l in ref.stdout.splitlines() if l.startswith("{")]
+        want = harness_rows(timeout=600, method=method, rng=tag, kernel=kernel, NTPB=NTPB, NB=NB, N=N, repeat=2)
         ours = subprocess.run([matrix_exe, name, tag, str(NTPB), str(NB), str(N)], capture_output=True, text=True, timeout=600)
         assert ours.returncode == 0, ours.stdout[-400:] + ours.stderr[-400:]
         got = [json.loads(l) for l in ours.stdout.splitlines() if l.startswith("{")]

@@ -9,14 +9,11 @@ The CPU oracle's EM takes cuRAND's HOST branches (expf/logf instead of ex2/lg2.a
 accept/reject decision differs between host and device: host-vs-device EM parity is per-path for the
 overwhelming majority of paths and statistical in aggregate.
 """
-import json
-import os
-import subprocess
-
 import numpy as np
 import pytest
 
 from oracle import oracle as o
+from ref_build import harness_rows
 
 pytestmark = pytest.mark.gpu
 
@@ -41,14 +38,7 @@ def em_engine_n(n, N, **kw):
 
 
 def _ref_cuda(**flags):
-    exe = o.REF_HARNESS_PATH
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/nmch_ref_harness not shipped")
-    cmd = [exe]
-    for k, v in flags.items():
-        cmd += [f"--{k}", str(v)]
-    out = subprocess.run(cmd, check=True, capture_output=True, text=True, timeout=900).stdout
-    return [json.loads(l) for l in out.splitlines() if l.startswith("{")]
+    return harness_rows(timeout=900, **flags)
 
 
 def _rel(a, b):

@@ -8,14 +8,11 @@ Bars (BASELINE.json north_star):
   * native Philox mode: within 3 standard errors of the oracle / reference and of the semi-analytic
     Heston price (+ the O(dt) Euler scheme bias the oracle itself shows).
 """
-import json
-import os
-import subprocess
-
 import numpy as np
 import pytest
 
 from oracle import oracle as o
+from ref_build import harness_rows
 
 pytestmark = pytest.mark.gpu
 
@@ -92,14 +89,7 @@ def test_compat_shard_offsets_select_subsequences():
 # compat modes vs the reference's CUDA build
 # ---------------------------------------------------------------------------------------------
 def _ref_cuda(plus_floor=False, **flags):
-    exe = o.REF_HARNESS_PLUS_PATH if plus_floor else o.REF_HARNESS_PATH
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/nmch_ref_harness[_plus] not shipped")
-    cmd = [exe]
-    for k, v in flags.items():
-        cmd += [f"--{k}", str(v)]
-    out = subprocess.run(cmd, check=True, capture_output=True, text=True, timeout=600).stdout
-    return [json.loads(l) for l in out.splitlines() if l.startswith("{")]
+    return harness_rows(plus_floor=plus_floor, timeout=600, **flags)
 
 
 def _rel(a, b):

@@ -8,7 +8,7 @@ import subprocess
 
 import pytest
 
-from oracle import oracle as o
+from ref_build import harness_rows
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -28,14 +28,7 @@ def _ours(*args):
 
 
 def _ref(**flags):
-    if not os.path.exists(o.REF_HARNESS_PATH):
-        pytest.skip("oracle/_ref/nmch_ref_harness not shipped")
-    cmd = [o.REF_HARNESS_PATH]
-    for k, v in flags.items():
-        cmd += [f"--{k}", str(v)]
-    out = subprocess.run(cmd, check=True, capture_output=True, text=True, timeout=600).stdout
-    # the reference's get_err() is NaN under its own K1 quirk and printf writes "-nan": not JSON
-    return [json.loads(l.replace("-nan", "NaN").replace(" nan", " NaN")) for l in out.splitlines() if l.startswith("{")]
+    return harness_rows(timeout=600, **flags)
 
 
 @pytest.mark.parametrize("method,N", [("fe", 200), ("em", 100)])
