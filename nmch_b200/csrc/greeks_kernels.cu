@@ -7,6 +7,7 @@
 //   leaves S_T, V_T and dS_T/dv_0 in HBM (12 bytes per path) and reduces the K = S_0 payoff moments like every path kernel.
 // strike_greeks_kernel: folds the two terminal arrays per strike: payoff moments, delta = 1{S_T > K} S_T / S_0,
 //   vega = 1{S_T > K} dS_T/dv_0 and its square (for the standard error), through the deterministic ticket reduction.
+//   A NaN path makes the strike's payoff, delta and vega sums NaN (DESIGN.md row A3); the in-the-money count stays a count.
 #include "fe_step.cuh"
 #include "kernels.cuh"
 
@@ -108,14 +109,18 @@ constexpr int kGreekBlocks = 296;           // 2 per SM, contiguous slices, 16-b
 __device__ __forceinline__ void greek_fold(float s, float b, float K, float inv_S0, double &pay, double &pay2,
                                            double &delta, double &itm, double &vega, double &vega2)
 {
-    const float p = fmaxf(s - K, 0.0f);
-    pay += (double)p;
-    pay2 += (double)p * (double)p;
+    const double p = payoff_or_nan(s, K);
+    pay += p;
+    pay2 += p * p;
     if (s > K) {
         delta += (double)(s * inv_S0);
         itm += 1.0;
         vega += (double)b;
         vega2 += (double)b * (double)b;
+    } else if (s != s) {                                     // a NaN path: carried into delta and vega too
+        delta += (double)s;
+        vega += (double)s;
+        vega2 += (double)s;
     }
 }
 

@@ -3,7 +3,8 @@
 // The path kernels leave S_T of every local path in HBM (4 bytes per path; 64 MB at 2^24 paths, which stays in
 // the 126 MB L2 between the two kernels).  This kernel folds them per strike: block (x, j) reduces a slice of the
 // paths for strike j and writes two moment pairs -- (payoff, payoff^2) as reduction slot 2j and (delta, in-the-money
-// count) as slot 2j+1 -- through the same deterministic FP64 ticket reduction as the path kernels.
+// count) as slot 2j+1 -- through the same deterministic FP64 ticket reduction as the path kernels.  A NaN path makes the
+// strike's payoff and delta sums NaN, as in the path kernels (payoff_or_nan, DESIGN.md row A3); the count stays a count.
 #include "kernels.cuh"
 
 namespace nmchb {
@@ -26,24 +27,28 @@ strike_moments_kernel(const float *__restrict__ S, unsigned long long n, const f
         const float v[4] = {s.x, s.y, s.z, s.w};
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
-            const float p = fmaxf(v[q] - K, 0.0f);
-            pay += (double)p;
-            pay2 += (double)p * (double)p;
+            const double p = payoff_or_nan(v[q], K);
+            pay += p;
+            pay2 += p * p;
             if (v[q] > K) {
                 delta += (double)(v[q] * inv_S0);
                 itm += 1.0;
+            } else if (v[q] != v[q]) {                       // a NaN path: carried into delta too
+                delta += (double)v[q];
             }
         }
     }
     if (blockIdx.x == 0) {                                   // ragged tail
         for (unsigned long long i = n4 * 4ull + threadIdx.x; i < n; i += blockDim.x) {
             const float v = S[i];
-            const float p = fmaxf(v - K, 0.0f);
-            pay += (double)p;
-            pay2 += (double)p * (double)p;
+            const double p = payoff_or_nan(v, K);
+            pay += p;
+            pay2 += p * p;
             if (v > K) {
                 delta += (double)(v * inv_S0);
                 itm += 1.0;
+            } else if (v != v) {
+                delta += (double)v;
             }
         }
     }

@@ -133,6 +133,14 @@ class Engine:
         return [{"strike": m.strike, "moments": Moments(m.sum_payoff, m.sum_payoff_sq, m.n_paths, m.exec_ms),
                  "delta": m.sum_delta / m.n_paths, "itm": m.sum_itm / m.n_paths} for m in out]
 
+    def compute_strikes_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
+        """Enqueue compute_strikes() on a caller stream; raw sums land in device memory (4 doubles per strike:
+        payoff, payoff^2, delta, in-the-money count)."""
+        strikes = np.ascontiguousarray(strikes, np.float32)
+        capi.check(self._lib.nmch_engine_compute_strikes_async(self._h, C.c_void_p(stream_ptr),
+                                                               strikes.ctypes.data_as(C.POINTER(C.c_float)),
+                                                               len(strikes), C.c_void_p(d_moments_ptr)))
+
     def compute_greeks(self, strikes):
         """compute_strikes() plus the pathwise vega d E[(S_T - K)^+] / d v_0 (FE, native Philox stream only)."""
         strikes = np.ascontiguousarray(strikes, np.float32)
@@ -140,6 +148,14 @@ class Engine:
         capi.check(self._lib.nmch_engine_compute_greeks(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
                                                         len(strikes), out))
         return _greek_rows(out)
+
+    def compute_greeks_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
+        """Enqueue compute_greeks() on a caller stream; raw sums land in device memory (6 doubles per strike:
+        payoff, payoff^2, delta, in-the-money count, vega, vega^2)."""
+        strikes = np.ascontiguousarray(strikes, np.float32)
+        capi.check(self._lib.nmch_engine_compute_greeks_async(self._h, C.c_void_p(stream_ptr),
+                                                              strikes.ctypes.data_as(C.POINTER(C.c_float)),
+                                                              len(strikes), C.c_void_p(d_moments_ptr)))
 
     def check(self) -> None:
         """Synchronise and, in the checked build, sweep the guard bands / surface a failed device assert."""
