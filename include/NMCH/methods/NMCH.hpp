@@ -65,6 +65,12 @@ public:
        only: the tangent rides the native Euler step; any other method / stream fails like every engine error). */
     float compute_greeks(int n_strikes, const float *strikes, float *price_out, float *price_squared_out, float *delta_out,
                          float *vega_out, float *vega_err_out);
+    /* The same pass with the pathwise sensitivities d E[(S_T-K)^+] / dp for p = v_0, kappa, theta, sigma, rho (in the
+       NMCH_SENS_* order of nmch_b200.h) and their standard errors: sens_out and sens_err_out hold NMCH_SENS_COUNT
+       values per strike, strike after strike (may be null).  FE on the native Philox stream with |rho| < 1 only; any
+       other method / stream fails like every engine error. */
+    float compute_sensitivities(int n_strikes, const float *strikes, float *price_out, float *price_squared_out,
+                                float *delta_out, float *sens_out, float *sens_err_out);
 
     virtual ~NMCH();
 

@@ -150,6 +150,40 @@ int nmch_engine_compute_greeks(nmch_engine_t *e, const float *strikes, int n_str
 int nmch_engine_compute_greeks_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
                                      double *d_moments);
 
+/* ---- ... and the pathwise sensitivities to every Heston parameter (no reference equivalent): the same pass carries
+ * the tangent of every path in five directions p = v_0, kappa, theta, sigma, rho at once, so one pass returns the full
+ * gradient of the FE-discretised, undiscounted price E[(S_T - K)^+] (the convention of compute_greeks) per strike:
+ *   sum_sens[p] = sum 1{S_T > K} dS_T/dp,   sum_sens_sq[p] = sum (1{S_T > K} dS_T/dp)^2   (for the standard error).
+ * The derivative is that of the FE map in the mathematical parameters (the host folds dt, kappa theta dt, ... in
+ * double; their derivatives are folded the same way), not of the float32 rounding of that folding.  sum_sens[NMCH_SENS_V0]
+ * and the four strike sums equal compute_greeks' and compute_strikes' bit for bit.  FE on the native Philox stream only;
+ * other methods / stream modes, n_strikes outside 1..NMCH_MAX_STRIKES and |rho| >= 1 (where d sqrt(1 - rho^2) / d rho is
+ * infinite) return NMCH_ERR_ARG and leave the engine as it was.  Streams advance exactly as for compute(). */
+#define NMCH_SENS_V0    0
+#define NMCH_SENS_KAPPA 1     /* the mean-reversion speed k of nmch_params_t */
+#define NMCH_SENS_THETA 2
+#define NMCH_SENS_SIGMA 3
+#define NMCH_SENS_RHO   4
+#define NMCH_SENS_COUNT 5
+typedef struct {
+    float  strike;
+    double sum_payoff;        /* sum (S_T - K)^+                      */
+    double sum_payoff_sq;     /* sum ((S_T - K)^+)^2                  */
+    double sum_delta;         /* sum 1{S_T > K} S_T / S_0             */
+    double sum_itm;           /* sum 1{S_T > K}                       */
+    double sum_sens[NMCH_SENS_COUNT];      /* sum 1{S_T > K} dS_T/dp, p in NMCH_SENS_* order */
+    double sum_sens_sq[NMCH_SENS_COUNT];   /* sum (1{S_T > K} dS_T/dp)^2          */
+    unsigned long long n_paths;
+    float  exec_ms;
+} nmch_sensitivity_moments_t;
+int nmch_engine_compute_sensitivities(nmch_engine_t *e, const float *strikes, int n_strikes,
+                                      nmch_sensitivity_moments_t *out);
+/* stream form: 14*n_strikes raw sums per strike into DEVICE memory, in the order
+ * {payoff, payoff^2, delta, itm, sens[v_0], sens_sq[v_0], sens[kappa], sens_sq[kappa], sens[theta], sens_sq[theta],
+ *  sens[sigma], sens_sq[sigma], sens[rho], sens_sq[rho]} */
+int nmch_engine_compute_sensitivities_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
+                                            double *d_moments);
+
 /* finalize() (NMCH_FE.cu:326-331); idempotent here (the reference double-frees) */
 int nmch_engine_finalize(nmch_engine_t *e);
 void nmch_engine_destroy(nmch_engine_t *e);
@@ -190,6 +224,8 @@ int nmch_group_finalize(nmch_group_t *g);
 void nmch_group_destroy(nmch_group_t *g);
 int nmch_group_compute_strikes(nmch_group_t *g, const float *strikes, int n_strikes, nmch_strike_moments_t *out);
 int nmch_group_compute_greeks(nmch_group_t *g, const float *strikes, int n_strikes, nmch_greek_moments_t *out);
+/* one allreduce of 14*n_strikes doubles */
+int nmch_group_compute_sensitivities(nmch_group_t *g, const float *strikes, int n_strikes, nmch_sensitivity_moments_t *out);
 float nmch_group_init_ms(const nmch_group_t *g);
 int nmch_group_size(const nmch_group_t *g);
 

@@ -40,6 +40,17 @@ class NmchGreekMoments(C.Structure):
                 ("n_paths", C.c_ulonglong), ("exec_ms", C.c_float)]
 
 
+# direction order of the sensitivity sums (NMCH_SENS_* of include/nmch_b200.h)
+SENS_V0, SENS_KAPPA, SENS_THETA, SENS_SIGMA, SENS_RHO, SENS_COUNT = 0, 1, 2, 3, 4, 5
+SENS_NAMES = ("v0", "kappa", "theta", "sigma", "rho")
+
+
+class NmchSensitivityMoments(C.Structure):
+    _fields_ = [("strike", C.c_float), ("sum_payoff", C.c_double), ("sum_payoff_sq", C.c_double),
+                ("sum_delta", C.c_double), ("sum_itm", C.c_double), ("sum_sens", C.c_double * SENS_COUNT),
+                ("sum_sens_sq", C.c_double * SENS_COUNT), ("n_paths", C.c_ulonglong), ("exec_ms", C.c_float)]
+
+
 class NmchLaunchInfo(C.Structure):
     _fields_ = [("grid_x", C.c_int), ("grid_y", C.c_int), ("block_threads", C.c_int),
                 ("paths_per_thread", C.c_int), ("regs_per_thread", C.c_int), ("sm_count", C.c_int),
@@ -51,6 +62,7 @@ EXPORTS = [
     "nmch_engine_compute_async", "nmch_engine_explore", "nmch_engine_explore_async",
     "nmch_engine_compute_paths", "nmch_engine_compute_strikes", "nmch_engine_compute_strikes_async",
     "nmch_engine_compute_greeks", "nmch_engine_compute_greeks_async", "nmch_group_compute_greeks",
+    "nmch_engine_compute_sensitivities", "nmch_engine_compute_sensitivities_async", "nmch_group_compute_sensitivities",
     "nmch_engine_finalize", "nmch_engine_destroy", "nmch_engine_init_ms", "nmch_engine_check", "nmch_checked_build", "nmch_checked_selftest",
     "nmch_engine_launch_info", "nmch_group_create", "nmch_group_init", "nmch_group_set_params", "nmch_group_compute",
     "nmch_group_explore", "nmch_group_compute_strikes", "nmch_group_finalize", "nmch_group_destroy", "nmch_group_init_ms", "nmch_group_size",
@@ -91,6 +103,9 @@ def load() -> C.CDLL:
     L.nmch_engine_compute_greeks.argtypes = [vp, f32p, C.c_int, C.POINTER(NmchGreekMoments)]
     L.nmch_engine_compute_greeks_async.argtypes = [vp, vp, f32p, C.c_int, vp]
     L.nmch_group_compute_greeks.argtypes = [vp, f32p, C.c_int, C.POINTER(NmchGreekMoments)]
+    L.nmch_engine_compute_sensitivities.argtypes = [vp, f32p, C.c_int, C.POINTER(NmchSensitivityMoments)]
+    L.nmch_engine_compute_sensitivities_async.argtypes = [vp, vp, f32p, C.c_int, vp]
+    L.nmch_group_compute_sensitivities.argtypes = [vp, f32p, C.c_int, C.POINTER(NmchSensitivityMoments)]
     L.nmch_engine_check.argtypes = [vp]
     L.nmch_checked_selftest.argtypes = [vp]
     L.nmch_engine_finalize.argtypes = [vp]

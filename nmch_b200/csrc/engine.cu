@@ -717,26 +717,52 @@ int nmch_engine_compute_strikes_async(nmch_engine_t *e, void *cuda_stream, const
     return strikes_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, d_moments);
 }
 
-// ---- strike vector with pathwise delta and vega (FE, native Philox stream) ------------------------------------------
-static int greeks_launch(nmch_engine *e, cudaStream_t stream, const float *strikes, int n_strikes, double *d_out6)
+// ---- strike vector with pathwise delta and vega / sensitivities (FE, native Philox stream) ---------------------------
+// The derivatives of the folded step constants in kappa, theta, sigma and rho (fe_step.cuh), in double, rounded once.
+static TangentFold fold_tangent(const nmch_params_t &p)
+{
+    const double dt = (double)(p.T / (float)p.N);                 // as fold_fe_point forms it
+    const double sdc = std::sqrt(dt) * 1.1774100225154747;         // sqrt(dt) sqrt(2 ln 2)
+    const double rho = (double)p.rho;
+    TangentFold tf;
+    tf.dva_k = (float)(-dt);
+    tf.dvb_k = (float)((double)p.theta * dt);
+    tf.dvb_t = (float)((double)p.k * dt);
+    tf.dvs_s = (float)sdc;
+    tf.dzr_r = (float)sdc;
+    tf.dzc_r = (float)(-rho / std::sqrt(1.0 - rho * rho) * sdc);
+    return tf;
+}
+
+// The native FE pass with the tangent in n_dirs directions (1: compute_greeks, 5: compute_sensitivities), then the fold
+// of 4 + 2 n_dirs raw sums per strike into d_out.
+static int greeks_launch(nmch_engine *e, cudaStream_t stream, const float *strikes, int n_strikes, int n_dirs, double *d_out)
 {
     const nmch_params_t &p = e->p;
-    if (p.method != NMCH_METHOD_FE || p.rng != NMCH_RNG_PHILOX)
-        return fail(NMCH_ERR_ARG, "compute_greeks: the pathwise tangent is carried by the native FE step (method FE, rng PHILOX)");
+    const char *what = n_dirs == 1 ? "compute_greeks" : "compute_sensitivities";
+    if (p.method != NMCH_METHOD_FE || p.rng != NMCH_RNG_PHILOX) {
+        char buf[160];
+        std::snprintf(buf, sizeof buf, "%s: the pathwise tangent is carried by the native FE step (method FE, rng PHILOX)", what);
+        return fail(NMCH_ERR_ARG, buf);
+    }
+    if (n_dirs > 1 && !(std::fabs(p.rho) < 1.0f))      // also refuses a NaN rho
+        return fail(NMCH_ERR_ARG, "compute_sensitivities: needs |rho| < 1 (d sqrt(1 - rho^2) / d rho is infinite at |rho| = 1)");
     int rc = ensure_sv(e, (size_t)e->n_local);
     if (rc) return rc;
-    if ((size_t)e->n_local > e->t_cap) {
+    const size_t t_need = n_dirs == 1 ? (size_t)e->n_local : (size_t)n_dirs * (size_t)tangent_stride(e->n_local);
+    if (t_need > e->t_cap) {
         engine_dev_free(e, e->d_T);
         e->d_T = nullptr;
         e->t_cap = 0;
-        CU_TRY(engine_dev_malloc(e, (void **)&e->d_T, (size_t)e->n_local * sizeof(float), "dS_T/dv_0"));
-        e->t_cap = (size_t)e->n_local;
+        CU_TRY(engine_dev_malloc(e, (void **)&e->d_T, t_need * sizeof(float), "dS_T/dp"));
+        e->t_cap = t_need;
     }
-    // reduction slots: 0 = the path kernel's own K = S_0 moments, 1 + 3j .. 3 + 3j = strike j (payoff, delta, vega)
-    const size_t slots = 1 + 3 * (size_t)n_strikes;
+    // reduction slots: 0 = the path kernel's own K = S_0 moments, then 2 + n_dirs per strike (payoff, delta, one per
+    // direction)
+    const size_t slots = 1 + (size_t)(2 + n_dirs) * (size_t)n_strikes;
     rc = ensure_buffers(e, slots, (size_t)greek_blocks_per_slot(), (size_t)n_strikes * sizeof(float));
     if (rc) return rc;
-    const unsigned long long tile = (unsigned long long)tangent_tile_paths();
+    const unsigned long long tile = (unsigned long long)tangent_tile_paths(n_dirs);
     const unsigned long long bpp = (e->n_local + tile - 1ull) / tile;
     if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
     rc = ensure_buffers(e, 1, (size_t)bpp, 0);
@@ -745,12 +771,14 @@ static int greeks_launch(nmch_engine *e, cudaStream_t stream, const float *strik
     CU_TRY(cudaStreamSynchronize(stream));                     // `strikes` is caller memory of unknown lifetime
     FeLaunch L;
     fill_fe_launch(e, L, 1, (int)bpp, 1);
+    const TangentFold tf = fold_tangent(p);
     ReduceBuffers rb0{e->d_partials, e->d_tickets, e->h_out_dev};
-    CU_TRY(launch_fe_tangent(L, p.floor, rb0, e->d_S, e->d_V, e->d_T, stream, &e->kinfo));
+    CU_TRY(launch_fe_tangent(L, p.floor, n_dirs, tf, rb0, e->d_S, e->d_V, e->d_T, stream, &e->kinfo));
     e->draw_offset += 2ull * (unsigned long long)p.N;          // the stream advances like one compute()
     // same stream: the path kernel (and its use of the partial buffer) is complete before the fold starts
-    ReduceBuffers rb{e->d_partials, e->d_tickets + 1, d_out6};
-    CU_TRY(launch_strike_greeks(e->d_S, e->d_T, e->n_local, static_cast<const float *>(e->d_points), n_strikes, p.S_0, rb, stream));
+    ReduceBuffers rb{e->d_partials, e->d_tickets + 1, d_out};
+    CU_TRY(launch_strike_greeks(e->d_S, e->d_T, n_dirs, e->n_local, static_cast<const float *>(e->d_points), n_strikes,
+                                p.S_0, rb, stream));
     e->launches += 2;
     return NMCH_OK;
 }
@@ -765,7 +793,7 @@ int nmch_engine_compute_greeks(nmch_engine_t *e, const float *strikes, int n_str
     rc = ensure_buffers(e, 1 + 3 * (size_t)n_strikes, 1, 0);   // host-visible result buffer large enough
     if (rc) return rc;
     CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = greeks_launch(e, e->stream, strikes, n_strikes, e->h_out_dev + 2);
+    rc = greeks_launch(e, e->stream, strikes, n_strikes, 1, e->h_out_dev + 2);
     if (rc) return rc;
     CU_TRY(cudaEventRecord(e->ev1, e->stream));
     CU_TRY(cudaEventSynchronize(e->ev1));
@@ -786,7 +814,41 @@ int nmch_engine_compute_greeks_async(nmch_engine_t *e, void *cuda_stream, const 
     if (!strikes || !d_moments || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
     DeviceGuard guard(e->device);
     if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    return greeks_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, d_moments);
+    return greeks_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, 1, d_moments);
+}
+
+int nmch_engine_compute_sensitivities(nmch_engine_t *e, const float *strikes, int n_strikes,
+                                      nmch_sensitivity_moments_t *out)
+{
+    int rc = check_ready(e);
+    if (rc) return rc;
+    if (!strikes || !out || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
+    DeviceGuard guard(e->device);
+    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
+    constexpr int kPer = 4 + 2 * NMCH_SENS_COUNT;
+    rc = ensure_buffers(e, 1 + (size_t)(kPer / 2) * (size_t)n_strikes, 1, 0);   // host-visible result buffer large enough
+    if (rc) return rc;
+    CU_TRY(cudaEventRecord(e->ev0, e->stream));
+    rc = greeks_launch(e, e->stream, strikes, n_strikes, NMCH_SENS_COUNT, e->h_out_dev + 2);
+    if (rc) return rc;
+    CU_TRY(cudaEventRecord(e->ev1, e->stream));
+    CU_TRY(cudaEventSynchronize(e->ev1));
+    float ms = 0.0f;
+    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
+    for (int j = 0; j < n_strikes; ++j)
+        sensitivity_unpack(e->h_out + 2 + kPer * (size_t)j, strikes[j], e->n_local, ms, &out[j]);
+    return engine_check_guards(e);
+}
+
+int nmch_engine_compute_sensitivities_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
+                                            double *d_moments)
+{
+    int rc = check_ready(e);
+    if (rc) return rc;
+    if (!strikes || !d_moments || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
+    DeviceGuard guard(e->device);
+    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
+    return greeks_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, NMCH_SENS_COUNT, d_moments);
 }
 
 int nmch_engine_finalize(nmch_engine_t *e)

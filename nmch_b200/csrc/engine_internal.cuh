@@ -39,7 +39,8 @@ struct nmch_engine {
     size_t points_cap = 0;
     float *d_S = nullptr, *d_V = nullptr;    // parity hook buffers
     size_t sv_cap = 0;
-    float *d_T = nullptr;                    // dS_T/dv_0 of every local path (compute_greeks)
+    float *d_T = nullptr;                    // dS_T/dp of every local path: v_0 (compute_greeks) or all five directions,
+                                             // tangent_stride(n_local) floats apart (compute_sensitivities)
     size_t t_cap = 0;
     // XORWOW-compat state
     nmchb::XorwowSkipTables *xtab = nullptr;
@@ -75,5 +76,25 @@ int mrg_compat_init(nmch_engine *e);
 cudaError_t launch_fe_compat_mrg(const FeLaunch &L, int floor_kind, const RawPoint *d_pts, void *states,
                                  ReduceBuffers rb, float *S_out, float *V_out, cudaStream_t stream, KernelInfo *info);
 void em_release(nmch_engine *e);
+
+static_assert(NMCH_SENS_COUNT == kNumDirs && NMCH_SENS_V0 == kDirV0 && NMCH_SENS_KAPPA == kDirKappa &&
+                  NMCH_SENS_THETA == kDirTheta && NMCH_SENS_SIGMA == kDirSigma && NMCH_SENS_RHO == kDirRho,
+              "the header's direction order is the kernels' order");
+// one strike's 14 raw sums (the layout of nmch_engine_compute_sensitivities_async) into the public struct
+inline void sensitivity_unpack(const double *m, float strike, unsigned long long n_paths, float ms,
+                               nmch_sensitivity_moments_t *out)
+{
+    out->strike = strike;
+    out->sum_payoff = m[0];
+    out->sum_payoff_sq = m[1];
+    out->sum_delta = m[2];
+    out->sum_itm = m[3];
+    for (int d = 0; d < NMCH_SENS_COUNT; ++d) {
+        out->sum_sens[d] = m[4 + 2 * d];
+        out->sum_sens_sq[d] = m[5 + 2 * d];
+    }
+    out->n_paths = n_paths;
+    out->exec_ms = ms;
+}
 
 }  // namespace nmchb

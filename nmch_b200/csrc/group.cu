@@ -265,7 +265,8 @@ int nmch_group_explore(nmch_group_t *g, const float *k, const float *theta, cons
     return run_points(g, k, theta, sigma, n_points, out);
 }
 
-// per strike `per` doubles of raw sums: 4 (payoff, payoff^2, delta, itm) or 6 (+ vega, vega^2; FE native stream only)
+// per strike `per` doubles of raw sums: 4 (payoff, payoff^2, delta, itm), 6 (+ vega, vega^2) or 14 (+ five sensitivities
+// and their squares); the last two FE native stream only
 static int group_strikes_impl(nmch_group_t *g, const float *strikes, int n_strikes, int per, float *ms_out)
 {
     if (!g || !g->inited) return engine_fail(NMCH_ERR_STATE, "group not initialised");
@@ -277,8 +278,9 @@ static int group_strikes_impl(nmch_group_t *g, const float *strikes, int n_strik
     for (int i = 0; i < g->n; ++i) {
         GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
         GROUP_CU_TRY(cudaEventRecord(g->ev0[i], g->stream[i]));
-        rc = per == 6 ? nmch_engine_compute_greeks_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i])
-                      : nmch_engine_compute_strikes_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i]);
+        rc = per == 14 ? nmch_engine_compute_sensitivities_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i])
+           : per == 6  ? nmch_engine_compute_greeks_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i])
+                       : nmch_engine_compute_strikes_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i]);
         if (rc) return rc;
     }
     if (g->n > 1) {
@@ -330,6 +332,17 @@ int nmch_group_compute_greeks(nmch_group_t *g, const float *strikes, int n_strik
         const double *m = g->h_mom + 6 * (size_t)j;
         out[j] = nmch_greek_moments_t{strikes[j], m[0], m[1], m[2], m[3], m[4], m[5], g->n_paths, ms};
     }
+    return NMCH_OK;
+}
+
+int nmch_group_compute_sensitivities(nmch_group_t *g, const float *strikes, int n_strikes, nmch_sensitivity_moments_t *out)
+{
+    if (!out) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
+    constexpr int kPer = 4 + 2 * NMCH_SENS_COUNT;
+    float ms = 0.0f;
+    const int rc = group_strikes_impl(g, strikes, n_strikes, kPer, &ms);
+    if (rc) return rc;
+    for (int j = 0; j < n_strikes; ++j) nmchb::sensitivity_unpack(g->h_mom + kPer * (size_t)j, strikes[j], g->n_paths, ms, &out[j]);
     return NMCH_OK;
 }
 

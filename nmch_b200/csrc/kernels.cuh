@@ -49,6 +49,21 @@ struct FeLaunch {
     RawPoint raw0;
 };
 
+// Directions of the pathwise tangent, in the order of nmch_sensitivity_moments_t (NMCH_SENS_V0 .. NMCH_SENS_RHO).
+constexpr int kDirV0 = 0, kDirKappa = 1, kDirTheta = 2, kDirSigma = 3, kDirRho = 4, kNumDirs = 5;
+
+// Derivatives of the folded step constants in the directions kappa, theta, sigma and rho (fold_tangent: double on the
+// host, rounded once).  They are taken of the mathematical FE map (va = 1 - k dt, vb = k theta dt, vs = sigma sqrt(dt) c0,
+// zr = rho sqrt(dt) c0, zc = sqrt(1 - rho^2) sqrt(dt) c0), not of the float32 rounding of the folding.
+struct TangentFold {
+    float dva_k;                        // d va / d kappa = -dt
+    float dvb_k;                        // d vb / d kappa = theta dt
+    float dvb_t;                        // d vb / d theta = kappa dt
+    float dvs_s;                        // d vs / d sigma = sqrt(dt) c0 (not vs / sigma: sigma = 0 is a valid point)
+    float dzr_r;                        // d zr / d rho   = sqrt(dt) c0
+    float dzc_r;                        // d zc / d rho   = -rho / sqrt(1 - rho^2) sqrt(dt) c0
+};
+
 struct ReduceBuffers {
     double2      *partials;             // [n_points][blocks_per_point]
     unsigned int *tickets;              // [n_points], zero between launches
@@ -90,14 +105,17 @@ cudaError_t launch_strike_moments(const float *d_S, unsigned long long n_local, 
                                   float S0, ReduceBuffers rb, cudaStream_t stream);
 int strike_blocks_per_slot();
 
-// greeks_kernels.cu: native FE pass carrying the pathwise tangent in v_0 (leaves S_T, V_T, dS_T/dv_0 on the device), and
-// the per-strike fold of payoff / delta / vega: 3 reduction slots = 6 doubles per strike
-cudaError_t launch_fe_tangent(const FeLaunch &L, int floor_kind, ReduceBuffers rb, float *S_out, float *V_out, float *B_out,
-                              cudaStream_t stream, KernelInfo *info);
-cudaError_t launch_strike_greeks(const float *d_S, const float *d_B, unsigned long long n_local, const float *d_strikes,
-                                 int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream);
+// greeks_kernels.cu: native FE pass carrying the pathwise tangent in n_dirs = 1 (v_0) or 5 (v_0, kappa, theta, sigma,
+// rho; fe_step.cuh) directions (leaves S_T, V_T and dS_T/dp of every direction on the device), and the per-strike fold of
+// payoff / delta / sensitivities: 2 + n_dirs reduction slots = 4 + 2 n_dirs doubles per strike
+cudaError_t launch_fe_tangent(const FeLaunch &L, int floor_kind, int n_dirs, const TangentFold &tf, ReduceBuffers rb,
+                              float *S_out, float *V_out, float *B_out, cudaStream_t stream, KernelInfo *info);
+cudaError_t launch_strike_greeks(const float *d_S, const float *d_B, int n_dirs, unsigned long long n_local,
+                                 const float *d_strikes, int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream);
 int greek_blocks_per_slot();
-int tangent_tile_paths();                 // paths per block of fe_tangent_kernel
+int tangent_tile_paths(int n_dirs);       // paths per block of fe_tangent_kernel
+// floats between the tangent arrays of two directions: n_local rounded up to 16 bytes, so that every array takes float4 loads
+__host__ __device__ inline unsigned long long tangent_stride(unsigned long long n_local) { return (n_local + 3ull) & ~3ull; }
 
 // xorwow.cu
 struct XorwowSkipTables;                // device tables M_m^q, q = 1..3, m = 0..31

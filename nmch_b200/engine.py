@@ -59,6 +59,25 @@ def _greek_rows(out):
                      "vega_v0_se": (var / max(n - 1, 1)) ** 0.5})
     return rows
 
+
+def _sensitivity_rows(out):
+    """Per strike: the keys of compute_strikes() (payoff moments, delta, in-the-money share) and, for each parameter p of
+    capi.SENS_NAMES, the pathwise d E[(S_T - K)^+] / d p as "d_<p>" and its standard error as "d_<p>_se" (computed as
+    _greek_rows computes vega_v0 / vega_v0_se)."""
+    rows = []
+    for m in out:
+        n = m.n_paths
+        row = {"strike": m.strike, "moments": Moments(m.sum_payoff, m.sum_payoff_sq, n, m.exec_ms),
+               "delta": m.sum_delta / n, "itm": m.sum_itm / n}
+        for d, name in enumerate(capi.SENS_NAMES):
+            mean = m.sum_sens[d] / n
+            var = max(m.sum_sens_sq[d] / n - mean * mean, 0.0)
+            row[f"d_{name}"] = mean
+            row[f"d_{name}_se"] = (var / max(n - 1, 1)) ** 0.5
+        rows.append(row)
+    return rows
+
+
 class Engine:
     def __init__(self, NTPB=512, NB=512, T=1.0, S_0=1.0, v_0=0.1, r=0.0, k=0.5, rho=-0.7, theta=0.1, sigma=0.3,
                  N=1000, method=METHOD_FE, floor=FLOOR_ABS, rng=RNG_PHILOX, device=-1, n_paths=0, first_path=0,
@@ -157,6 +176,24 @@ class Engine:
                                                               strikes.ctypes.data_as(C.POINTER(C.c_float)),
                                                               len(strikes), C.c_void_p(d_moments_ptr)))
 
+    def compute_sensitivities(self, strikes):
+        """compute_strikes() plus the pathwise sensitivities of E[(S_T - K)^+] to v_0, kappa, theta, sigma and rho from
+        the same pass (FE, native Philox stream only; |rho| < 1).  Rows carry "d_v0", "d_kappa", "d_theta", "d_sigma",
+        "d_rho" and their standard errors "d_<p>_se"."""
+        strikes = np.ascontiguousarray(strikes, np.float32)
+        out = (capi.NmchSensitivityMoments * len(strikes))()
+        capi.check(self._lib.nmch_engine_compute_sensitivities(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
+                                                               len(strikes), out))
+        return _sensitivity_rows(out)
+
+    def compute_sensitivities_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
+        """Enqueue compute_sensitivities() on a caller stream; raw sums land in device memory (14 doubles per strike:
+        payoff, payoff^2, delta, in-the-money count, then sum and sum of squares for v_0, kappa, theta, sigma, rho)."""
+        strikes = np.ascontiguousarray(strikes, np.float32)
+        capi.check(self._lib.nmch_engine_compute_sensitivities_async(self._h, C.c_void_p(stream_ptr),
+                                                                     strikes.ctypes.data_as(C.POINTER(C.c_float)),
+                                                                     len(strikes), C.c_void_p(d_moments_ptr)))
+
     def check(self) -> None:
         """Synchronise and, in the checked build, sweep the guard bands / surface a failed device assert."""
         capi.check(self._lib.nmch_engine_check(self._h))
@@ -243,6 +280,13 @@ class Group:
         capi.check(self._lib.nmch_group_compute_greeks(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
                                                        len(strikes), out))
         return _greek_rows(out)
+
+    def compute_sensitivities(self, strikes):
+        strikes = np.ascontiguousarray(strikes, np.float32)
+        out = (capi.NmchSensitivityMoments * len(strikes))()
+        capi.check(self._lib.nmch_group_compute_sensitivities(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
+                                                              len(strikes), out))
+        return _sensitivity_rows(out)
 
     @property
     def size(self) -> int:

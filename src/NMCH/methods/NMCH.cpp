@@ -158,6 +158,30 @@ float NMCH<rnd_state>::compute_greeks(int n_strikes, const float *strikes, float
 }
 
 template <typename rnd_state>
+float NMCH<rnd_state>::compute_sensitivities(int n_strikes, const float *strikes, float *price_out, float *sq_out,
+                                             float *delta_out, float *sens_out, float *sens_err_out)
+{
+    if (!group) testNMCH(NMCH_ERR_STATE);
+    testNMCH(nmch_group_set_params(group, k, theta, sigma));
+    std::vector<nmch_sensitivity_moments_t> m((size_t)(n_strikes > 0 ? n_strikes : 0));
+    testNMCH(nmch_group_compute_sensitivities(group, strikes, n_strikes, m.data()));
+    for (int j = 0; j < n_strikes; ++j) {
+        const double n = (double)m[j].n_paths;
+        if (price_out) price_out[j] = (float)(m[j].sum_payoff / n);
+        if (sq_out) sq_out[j] = (float)(m[j].sum_payoff_sq / n);
+        if (delta_out) delta_out[j] = (float)(m[j].sum_delta / n);
+        for (int d = 0; d < NMCH_SENS_COUNT; ++d) {
+            const double mean = m[j].sum_sens[d] / n;
+            const double var = m[j].sum_sens_sq[d] / n - mean * mean;
+            if (sens_out) sens_out[(size_t)j * NMCH_SENS_COUNT + d] = (float)mean;
+            if (sens_err_out)
+                sens_err_out[(size_t)j * NMCH_SENS_COUNT + d] = (float)std::sqrt((var > 0.0 ? var : 0.0) / (n > 1.0 ? n - 1.0 : 1.0));
+        }
+    }
+    return n_strikes > 0 ? m[0].exec_ms : 0.0f;
+}
+
+template <typename rnd_state>
 void NMCH<rnd_state>::apply_legacy_k1_moment()
 {
     // reference FE_k1 / EM_k1: SR = payoff / n; VR = SR * SR / n; price_squared = sum VR = (sum payoff^2) / n^3

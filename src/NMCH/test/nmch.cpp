@@ -26,7 +26,7 @@ struct Options {
     float T = 1.0f, S_0 = 1.0f, v_0 = 0.1f, r = 0.0f, k = 0.5f, rho = -0.7, theta = 0.1f, sigma = 0.3f;
     unsigned long long seed = 1234;
     std::string method = "fe", g = "abs", rng = "philox", strikes;
-    bool json = false, legacy_k1 = false, vega = false;
+    bool json = false, legacy_k1 = false, vega = false, sensitivities = false;
 };
 
 void usage(const char *argv0)
@@ -57,6 +57,8 @@ void usage(const char *argv0)
     printf("  --paths-per-thread <int>  1, 2, 4 or 8 (default: auto)\n");
     printf("  --strikes <k1,k2,..>  Also price these strikes (and pathwise deltas) on a second pass of the streams\n");
     printf("  --vega                With --strikes: add the pathwise vega d price / d v_0 (fe, --rng philox only)\n");
+    printf("  --sensitivities       With --strikes: add the pathwise d price / d p and its std error for p = v_0, k, theta,\n");
+    printf("                        sigma, rho, all from the same pass (fe, --rng philox only, |rho| < 1)\n");
     printf("  --legacy-k1        Run the method's K1 class with the reference's K1 moment quirk (E[X^2] field = E[X^2]/n^2)\n");
     printf("  --json             Also print one JSON line with the raw moments\n");
 }
@@ -99,7 +101,18 @@ int run(const Options &o)
             p = q + 1;
         }
         std::vector<float> pr(ks.size()), sq(ks.size()), dl(ks.size());
-        if (o.vega) {
+        if (o.sensitivities) {
+            std::vector<float> sv(ks.size() * NMCH_SENS_COUNT), se(ks.size() * NMCH_SENS_COUNT);
+            const float ms = m.compute_sensitivities((int)ks.size(), ks.data(), pr.data(), sq.data(), dl.data(), sv.data(), se.data());
+            printf("strike, price, price_squared, delta, d_v0, d_v0_std_error, d_k, d_k_std_error, d_theta, d_theta_std_error, "
+                   "d_sigma, d_sigma_std_error, d_rho, d_rho_std_error   (one pass, %f ms)\n", ms);
+            for (size_t j = 0; j < ks.size(); ++j) {
+                printf("%f, %f, %f, %f", ks[j], pr[j], sq[j], dl[j]);
+                for (int d = 0; d < NMCH_SENS_COUNT; ++d)
+                    printf(", %f, %f", sv[j * NMCH_SENS_COUNT + d], se[j * NMCH_SENS_COUNT + d]);
+                printf("\n");
+            }
+        } else if (o.vega) {
             std::vector<float> vg(ks.size()), ve(ks.size());
             const float ms = m.compute_greeks((int)ks.size(), ks.data(), pr.data(), sq.data(), dl.data(), vg.data(), ve.data());
             printf("strike, price, price_squared, delta, vega_v0, vega_v0_std_error   (one pass, %f ms)\n", ms);
@@ -142,6 +155,7 @@ int main(int argc, char **argv)
         else if (strcmp(argv[i], "--json") == 0) o.json = true;
         else if (strcmp(argv[i], "--legacy-k1") == 0) o.legacy_k1 = true;
         else if (strcmp(argv[i], "--vega") == 0) o.vega = true;
+        else if (strcmp(argv[i], "--sensitivities") == 0) o.sensitivities = true;
         else if (strcmp(argv[i], "--help") == 0) { usage(argv[0]); return 0; }
     }
     if (o.rng != "philox" && o.rng != "xorwow" && o.rng != "philox-compat" && o.rng != "philox-dense" &&
