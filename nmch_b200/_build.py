@@ -19,7 +19,7 @@ BIN = os.path.join(ROOT, "bin")
 NVCC = os.environ.get("NVCC") or shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC"]
-CU_SOURCES = ["engine.cu", "fe_kernels.cu", "em_kernels.cu", "xorwow.cu", "group.cu", "strike_kernels.cu", "qe_kernels.cu", "greeks_kernels.cu"]
+CU_SOURCES = ["engine.cu", "fe_kernels.cu", "em_kernels.cu", "xorwow.cu", "group.cu", "qe_kernels.cu", "greeks_kernels.cu"]
 
 
 def _newer(target: str, deps) -> bool:

@@ -638,13 +638,12 @@ int em_launch_points(nmch_engine *e, cudaStream_t stream, const float *k, const 
         auto rank_of = [](const EmPoint &q) { return q.kind == kEmMixture ? 0 : (q.kind == kEmSplit ? 1 : 2); };
         std::stable_sort(pts.begin(), pts.end(), [&](const EmPoint &a, const EmPoint &b) { return rank_of(a) < rank_of(b); });
         const bool one_kind = pts.front().kind == pts.back().kind;
-        int rc = engine_ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(EmPoint));
+        int rc = engine_ensure_buffers(e, n_points, bpp);
         if (rc) return rc;
         const EmPoint *d_pts = nullptr;
         if (!own) {
-            err = cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(EmPoint), cudaMemcpyHostToDevice, stream);
-            if (err == cudaSuccess) err = cudaStreamSynchronize(stream);
-            if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "EM point upload", err);
+            rc = upload_records(e, stream, pts.data(), pts.size() * sizeof(EmPoint));
+            if (rc) return rc;
             d_pts = static_cast<const EmPoint *>(e->d_points);
         }
         EmLaunch L{};
@@ -690,15 +689,14 @@ int em_launch_points(nmch_engine *e, cudaStream_t stream, const float *k, const 
     }
     // compat modes
     bpp = (e->n_local + 255ull) / 256ull;
-    int rc = engine_ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(RawPoint));
+    int rc = engine_ensure_buffers(e, n_points, bpp);
     if (rc) return rc;
     const RawPoint *d_pts = nullptr;
     if (!own) {
         std::vector<RawPoint> pts(n_points);
         for (int i = 0; i < n_points; ++i) pts[i] = RawPoint{k[i], theta[i], sigma[i], 0.0f};
-        err = cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(RawPoint), cudaMemcpyHostToDevice, stream);
-        if (err == cudaSuccess) err = cudaStreamSynchronize(stream);
-        if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "EM point upload", err);
+        rc = upload_records(e, stream, pts.data(), pts.size() * sizeof(RawPoint));
+        if (rc) return rc;
         d_pts = static_cast<const RawPoint *>(e->d_points);
     }
     EmCompatLaunch L{};

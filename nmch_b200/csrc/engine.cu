@@ -192,7 +192,7 @@ void fill_fe_launch(const nmch_engine *e, FeLaunch &L, int n_points, int blocks_
     L.raw0 = RawPoint{p.k, p.theta, p.sigma, 0.0f};
 }
 
-int ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point, size_t point_bytes)
+int ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point)
 {
     const size_t need_partials = n_points * blocks_per_point;
     if (need_partials > e->partials_cap) {
@@ -220,13 +220,6 @@ int ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point, siz
         CU_TRY(cudaHostAlloc((void **)&e->h_out, 2 * n_points * sizeof(double), cudaHostAllocMapped));
         CU_TRY(cudaHostGetDevicePointer((void **)&e->h_out_dev, e->h_out, 0));
         e->out_cap = 2 * n_points;
-    }
-    if (point_bytes > e->points_cap) {
-        engine_dev_free(e, e->d_points);
-        e->d_points = nullptr;
-        e->points_cap = 0;
-        CU_TRY(engine_dev_malloc(e, &e->d_points, point_bytes, "points"));
-        e->points_cap = point_bytes;
     }
     return NMCH_OK;
 }
@@ -317,79 +310,55 @@ int launch_points(nmch_engine *e, cudaStream_t stream, const float *k, const flo
         if (rc) return rc;
     }
     if (p.method == NMCH_METHOD_FE) {
-        FeLaunch L;
+        const bool xorwow_fast = (p.rng == NMCH_RNG_XORWOW_FAST);
+        int P = 1, threads = 256, tiles_per_block = 1;
+        unsigned long long bpp = (e->n_local + 255ull) / 256ull;   // the XORWOW and MRG kernels: one path per thread
         if (native) {
-            int P = pick_paths_per_thread(e, n_points);
+            P = pick_paths_per_thread(e, n_points);
             if (exact && P > 2) P = 2;
             if (dense && P > 4) P = 4;
-            const int threads = dense ? 128 : e->threads;
+            threads = dense ? 128 : e->threads;
             const unsigned long long tile = (unsigned long long)P * threads;
             const unsigned long long tiles = (e->n_local + tile - 1) / tile;
             // keep the per-point partial list short when many points share the launch
-            int tiles_per_block = 1;
             if (n_points > 1 && tiles > 256ull) tiles_per_block = (int)((tiles + 255ull) / 256ull);
-            const unsigned long long bpp = (tiles + tiles_per_block - 1) / tiles_per_block;
-            if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
-            fill_fe_launch(e, L, n_points, (int)bpp, tiles_per_block);
-            int rc = ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(FePoint));
+            bpp = (tiles + tiles_per_block - 1) / tiles_per_block;
+        }
+        if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
+        FeLaunch L;
+        fill_fe_launch(e, L, n_points, (int)bpp, tiles_per_block);
+        int rc = ensure_buffers(e, n_points, bpp);
+        if (rc) return rc;
+        // Per-point records: the folded constants for the native step (XORWOW_FAST with the exact map of V), the raw
+        // (k, theta, sigma, 0) for the reference's IEEE arithmetic (Philox-compat) and the compat kernels' RawPoint, which
+        // has the same layout.
+        const void *d_pts = nullptr;
+        if (!own) {
+            const bool raw = exact || !(native || xorwow_fast);
+            std::vector<FePoint> pts(n_points);
+            for (int i = 0; i < n_points; ++i)
+                pts[i] = raw ? FePoint{k[i], theta[i], sigma[i], 0.0f} : fold_fe_point(p, k[i], theta[i], sigma[i], xorwow_fast);
+            rc = upload_records(e, stream, pts.data(), pts.size() * sizeof(FePoint));
             if (rc) return rc;
-            const FePoint *d_pts = nullptr;
-            if (!own) {
-                std::vector<FePoint> pts(n_points);
-                for (int i = 0; i < n_points; ++i)
-                    pts[i] = exact ? FePoint{k[i], theta[i], sigma[i], 0.0f} : fold_fe_point(p, k[i], theta[i], sigma[i]);
-                CU_TRY(cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(FePoint), cudaMemcpyHostToDevice, stream));
-                CU_TRY(cudaStreamSynchronize(stream));          // pts is a stack-lifetime staging buffer
-                d_pts = static_cast<const FePoint *>(e->d_points);
-            }
-            ReduceBuffers rb{e->d_partials, e->d_tickets, d_out};
-            if (dense)
-                CU_TRY(launch_fe_dense(L, p.floor, P, d_pts, rb, S_out, V_out, stream, &e->kinfo));
-            else
-                CU_TRY(launch_fe_philox(L, p.floor, P, threads, exact, d_pts, rb, S_out, V_out, stream, &e->kinfo));
-        } else if (p.rng == NMCH_RNG_XORWOW_FAST) {
-            // the XORWOW stream of the compat mode, the folded constants of the native mode
-            const unsigned long long bpp = (e->n_local + 255ull) / 256ull;
-            if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
-            fill_fe_launch(e, L, n_points, (int)bpp, 1);
-            int rc = ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(FePoint));
-            if (rc) return rc;
-            const FePoint *d_pts = nullptr;
-            if (!own) {
-                std::vector<FePoint> pts(n_points);
-                for (int i = 0; i < n_points; ++i) pts[i] = fold_fe_point(p, k[i], theta[i], sigma[i], true);
-                CU_TRY(cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(FePoint), cudaMemcpyHostToDevice, stream));
-                CU_TRY(cudaStreamSynchronize(stream));
-                d_pts = static_cast<const FePoint *>(e->d_points);
-            }
-            ReduceBuffers rb{e->d_partials, e->d_tickets, d_out};
+            d_pts = e->d_points;
+        }
+        const FePoint *fe_pts = static_cast<const FePoint *>(d_pts);
+        const RawPoint *raw_pts = static_cast<const RawPoint *>(d_pts);
+        ReduceBuffers rb{e->d_partials, e->d_tickets, d_out};
+        if (dense) {
+            CU_TRY(launch_fe_dense(L, p.floor, P, fe_pts, rb, S_out, V_out, stream, &e->kinfo));
+        } else if (native) {
+            CU_TRY(launch_fe_philox(L, p.floor, P, threads, exact, fe_pts, rb, S_out, V_out, stream, &e->kinfo));
+        } else if (p.rng == NMCH_RNG_MRG32K3A_COMPAT) {
+            CU_TRY(launch_fe_compat_mrg(L, p.floor, raw_pts, e->curand_states, rb, S_out, V_out, stream, &e->kinfo));
+        } else {
             const uint32_t *skip = nullptr;
             rc = plan_xorwow_chunks(e, stream, n_points, L, &skip);
             if (rc) return rc;
-            CU_TRY(launch_fe_xorwow_fast(L, p.floor, d_pts, e->xs, skip, rb, S_out, V_out, stream, &e->kinfo));
-        } else {
-            const unsigned long long bpp = (e->n_local + 255ull) / 256ull;
-            if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
-            fill_fe_launch(e, L, n_points, (int)bpp, 1);
-            int rc = ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(RawPoint));
-            if (rc) return rc;
-            const RawPoint *d_pts = nullptr;
-            if (!own) {
-                std::vector<RawPoint> pts(n_points);
-                for (int i = 0; i < n_points; ++i) pts[i] = RawPoint{k[i], theta[i], sigma[i], 0.0f};
-                CU_TRY(cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(RawPoint), cudaMemcpyHostToDevice, stream));
-                CU_TRY(cudaStreamSynchronize(stream));
-                d_pts = static_cast<const RawPoint *>(e->d_points);
-            }
-            ReduceBuffers rb{e->d_partials, e->d_tickets, d_out};
-            if (p.rng == NMCH_RNG_MRG32K3A_COMPAT) {
-                CU_TRY(launch_fe_compat_mrg(L, p.floor, d_pts, e->curand_states, rb, S_out, V_out, stream, &e->kinfo));
-            } else {
-                const uint32_t *skip = nullptr;
-                rc = plan_xorwow_chunks(e, stream, n_points, L, &skip);
-                if (rc) return rc;
-                CU_TRY(launch_fe_compat(L, p.floor, d_pts, e->xs, skip, rb, S_out, V_out, stream, &e->kinfo));
-            }
+            if (xorwow_fast)
+                CU_TRY(launch_fe_xorwow_fast(L, p.floor, fe_pts, e->xs, skip, rb, S_out, V_out, stream, &e->kinfo));
+            else
+                CU_TRY(launch_fe_compat(L, p.floor, raw_pts, e->xs, skip, rb, S_out, V_out, stream, &e->kinfo));
         }
         e->draw_offset += 2ull * (unsigned long long)p.N * (unsigned long long)n_points;
     } else if (p.method == NMCH_METHOD_EM) {
@@ -420,13 +389,153 @@ void fill_moments(const nmch_engine *e, const double *src, int n_points, float m
     }
 }
 
+// The blocking entry points: the engine's device current, a host-visible result buffer of n_slots reduction slots (2 doubles
+// each), launch(stream, d_out) timed on the engine's stream between ev0 and ev1, then unpack(h_out, exec_ms) and the guard
+// sweep of the checked build.
+template <class Launch, class Unpack>
+int blocking_call(nmch_engine *e, size_t n_slots, Launch launch, Unpack unpack)
+{
+    DeviceGuard guard(e->device);
+    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
+    int rc = ensure_buffers(e, n_slots, 1);
+    if (rc) return rc;
+    CU_TRY(cudaEventRecord(e->ev0, e->stream));
+    rc = launch(e->stream, e->h_out_dev);
+    if (rc) return rc;
+    CU_TRY(cudaEventRecord(e->ev1, e->stream));
+    CU_TRY(cudaEventSynchronize(e->ev1));
+    float ms = 0.0f;
+    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
+    unpack(static_cast<const double *>(e->h_out), ms);
+    return engine_check_guards(e);
+}
+
+int check_strike_call(const nmch_engine *e, const float *strikes, int n_strikes, const void *out)
+{
+    int rc = check_ready(e);
+    if (rc) return rc;
+    if (!strikes || !out || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
+    return NMCH_OK;
+}
+
+// The derivatives of the folded step constants in kappa, theta, sigma and rho (fe_step.cuh), in double, rounded once.
+TangentFold fold_tangent(const nmch_params_t &p)
+{
+    const double dt = (double)(p.T / (float)p.N);                 // as fold_fe_point forms it
+    const double sdc = std::sqrt(dt) * 1.1774100225154747;         // sqrt(dt) sqrt(2 ln 2)
+    const double rho = (double)p.rho;
+    TangentFold tf;
+    tf.dva_k = (float)(-dt);
+    tf.dvb_k = (float)((double)p.theta * dt);
+    tf.dvb_t = (float)((double)p.k * dt);
+    tf.dvs_s = (float)sdc;
+    tf.dzr_r = (float)sdc;
+    tf.dzc_r = (float)(-rho / std::sqrt(1.0 - rho * rho) * sdc);
+    return tf;
+}
+
+// One pass of the strike family on `stream`, shared by the blocking and the stream forms.  A path pass leaves S_T (and,
+// for n_dirs >= 1, dS_T/dp in n_dirs directions) on the device; strike_fold_kernel<n_dirs> then folds strike_doubles(n_dirs)
+// raw sums per strike into d_out.  n_dirs = 0 (compute_strikes) takes every method and stream; the tangent (1:
+// compute_greeks, 5: compute_sensitivities) is carried by the native FE step only.  Those refusals come first: a refused
+// call leaves the engine as it was.
+int strike_pass(nmch_engine *e, cudaStream_t stream, const float *strikes, int n_strikes, int n_dirs, double *d_out)
+{
+    const nmch_params_t &p = e->p;
+    if (n_dirs > 0 && (p.method != NMCH_METHOD_FE || p.rng != NMCH_RNG_PHILOX)) {
+        char buf[160];
+        std::snprintf(buf, sizeof buf, "%s: the pathwise tangent is carried by the native FE step (method FE, rng PHILOX)",
+                      n_dirs == 1 ? "compute_greeks" : "compute_sensitivities");
+        return fail(NMCH_ERR_ARG, buf);
+    }
+    if (n_dirs > 1 && !(std::fabs(p.rho) < 1.0f))      // also refuses a NaN rho
+        return fail(NMCH_ERR_ARG, "compute_sensitivities: needs |rho| < 1 (d sqrt(1 - rho^2) / d rho is infinite at |rho| = 1)");
+    int rc = ensure_sv(e, (size_t)e->n_local);
+    if (rc) return rc;
+    // reduction slots: 0 = the path kernel's own K = S_0 moments, then 2 + n_dirs per strike (payoff, delta, one per
+    // direction)
+    const size_t slots = 1 + (size_t)strike_doubles(n_dirs) / 2 * (size_t)n_strikes;
+    rc = ensure_buffers(e, slots, (size_t)strike_blocks_per_slot());
+    if (rc) return rc;
+    rc = upload_records(e, stream, strikes, (size_t)n_strikes * sizeof(float));
+    if (rc) return rc;
+    if (n_dirs == 0) {
+        rc = launch_points(e, stream, nullptr, nullptr, nullptr, 1, e->h_out_dev, e->d_S, e->d_V);
+        if (rc) return rc;
+    } else {
+        const size_t t_need = n_dirs == 1 ? (size_t)e->n_local : (size_t)n_dirs * (size_t)tangent_stride(e->n_local);
+        if (t_need > e->t_cap) {
+            engine_dev_free(e, e->d_T);
+            e->d_T = nullptr;
+            e->t_cap = 0;
+            CU_TRY(engine_dev_malloc(e, (void **)&e->d_T, t_need * sizeof(float), "dS_T/dp"));
+            e->t_cap = t_need;
+        }
+        const unsigned long long tile = (unsigned long long)tangent_tile_paths(n_dirs);
+        const unsigned long long bpp = (e->n_local + tile - 1ull) / tile;
+        if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
+        rc = ensure_buffers(e, 1, (size_t)bpp);
+        if (rc) return rc;
+        FeLaunch L;
+        fill_fe_launch(e, L, 1, (int)bpp, 1);
+        ReduceBuffers rb0{e->d_partials, e->d_tickets, e->h_out_dev};
+        CU_TRY(launch_fe_tangent(L, p.floor, n_dirs, fold_tangent(p), rb0, e->d_S, e->d_V, e->d_T, stream, &e->kinfo));
+        e->draw_offset += 2ull * (unsigned long long)p.N;          // the stream advances like one compute()
+        e->launches += 1;
+    }
+    // same stream: the path kernel (and its use of the partial buffer) is complete before the fold starts
+    ReduceBuffers rb{e->d_partials, e->d_tickets + 1, d_out};
+    CU_TRY(launch_strike_fold(e->d_S, e->d_T, n_dirs, e->n_local, static_cast<const float *>(e->d_points), n_strikes, p.S_0,
+                              rb, stream));
+    e->launches += 1;
+    return NMCH_OK;
+}
+
+// The blocking form of the strike family: n_dirs = 0, 1 or NMCH_SENS_COUNT, as the struct T carries.
+template <class T>
+int strike_call(nmch_engine *e, const float *strikes, int n_strikes, int n_dirs, T *out)
+{
+    const int rc = check_strike_call(e, strikes, n_strikes, out);
+    if (rc) return rc;
+    const size_t per = (size_t)strike_doubles(n_dirs);
+    return blocking_call(
+        e, 1 + per / 2 * (size_t)n_strikes,                     // slot 0: the path kernel's own K = S_0 moments
+        [&](cudaStream_t s, double *d_out) { return strike_pass(e, s, strikes, n_strikes, n_dirs, d_out + 2); },
+        [&](const double *h, float ms) {
+            for (int j = 0; j < n_strikes; ++j) strike_unpack(h + 2 + per * (size_t)j, strikes[j], e->n_local, ms, &out[j]);
+        });
+}
+
 }  // namespace
 
-// em_kernels.cu needs these engine internals
+// em_kernels.cu and qe_kernels.cu need these engine internals
 namespace nmchb {
-int engine_ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point, size_t point_bytes)
+int engine_ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point)
 {
-    return ensure_buffers(e, n_points, blocks_per_point, point_bytes);
+    return ensure_buffers(e, n_points, blocks_per_point);
+}
+
+int upload_records(nmch_engine *e, cudaStream_t stream, const void *host, size_t bytes)
+{
+    if (bytes > e->points_cap) {
+        engine_dev_free(e, e->d_points);
+        e->d_points = nullptr;
+        e->points_cap = 0;
+        CU_TRY(engine_dev_malloc(e, &e->d_points, bytes, "points"));
+        e->points_cap = bytes;
+    }
+    CU_TRY(cudaMemcpyAsync(e->d_points, host, bytes, cudaMemcpyHostToDevice, stream));
+    CU_TRY(cudaStreamSynchronize(stream));
+    return NMCH_OK;
+}
+
+int engine_strike_async(nmch_engine *e, void *cuda_stream, const float *strikes, int n_strikes, int n_dirs, double *d_out)
+{
+    const int rc = check_strike_call(e, strikes, n_strikes, d_out);
+    if (rc) return rc;
+    DeviceGuard guard(e->device);
+    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
+    return strike_pass(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, n_dirs, d_out);
 }
 }  // namespace nmchb
 
@@ -533,7 +642,7 @@ static int engine_init_impl(nmch_engine_t *e, unsigned long long seed)
         int rc = mrg_compat_init(e);
         if (rc) return rc;
     }
-    int rc = ensure_buffers(e, 1, 1, 0);
+    int rc = ensure_buffers(e, 1, 1);
     if (rc) return rc;
     CU_TRY(cudaEventRecord(e->ev1, e->stream));
     CU_TRY(cudaEventSynchronize(e->ev1));
@@ -569,19 +678,10 @@ int nmch_engine_compute(nmch_engine_t *e, nmch_moments_t *out)
     if (rc) return rc;
     if (!out) return fail(NMCH_ERR_ARG, "null output");
     NvtxRange range("nmch_engine_compute");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    rc = ensure_buffers(e, 1, 1, 0);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = launch_points(e, e->stream, nullptr, nullptr, nullptr, 1, e->h_out_dev, nullptr, nullptr);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev1, e->stream));
-    CU_TRY(cudaEventSynchronize(e->ev1));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
-    fill_moments(e, e->h_out, 1, ms, out);
-    return engine_check_guards(e);
+    return blocking_call(
+        e, 1,
+        [&](cudaStream_t s, double *d_out) { return launch_points(e, s, nullptr, nullptr, nullptr, 1, d_out, nullptr, nullptr); },
+        [&](const double *h, float ms) { fill_moments(e, h, 1, ms, out); });
 }
 
 int nmch_engine_compute_async(nmch_engine_t *e, void *cuda_stream, double *d_moments)
@@ -603,19 +703,10 @@ int nmch_engine_explore(nmch_engine_t *e, const float *k, const float *theta, co
     if (!k || !theta || !sigma || !out || n_points <= 0) return fail(NMCH_ERR_ARG, "bad exploration arguments");
     if (n_points > 65535) return fail(NMCH_ERR_ARG, "at most 65535 points per launch");
     NvtxRange range("nmch_engine_explore");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    rc = ensure_buffers(e, n_points, 1, 0);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = launch_points(e, e->stream, k, theta, sigma, n_points, e->h_out_dev, nullptr, nullptr);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev1, e->stream));
-    CU_TRY(cudaEventSynchronize(e->ev1));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
-    fill_moments(e, e->h_out, n_points, ms, out);
-    return engine_check_guards(e);
+    return blocking_call(
+        e, (size_t)n_points,
+        [&](cudaStream_t s, double *d_out) { return launch_points(e, s, k, theta, sigma, n_points, d_out, nullptr, nullptr); },
+        [&](const double *h, float ms) { fill_moments(e, h, n_points, ms, out); });
 }
 
 int nmch_engine_explore_async(nmch_engine_t *e, void *cuda_stream, const float *k, const float *theta,
@@ -642,7 +733,7 @@ int nmch_engine_compute_paths(nmch_engine_t *e, float *S_out, float *V_out, unsi
     if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
     rc = ensure_sv(e, (size_t)e->n_local);
     if (rc) return rc;
-    rc = ensure_buffers(e, 1, 1, 0);
+    rc = ensure_buffers(e, 1, 1);
     if (rc) return rc;
     CU_TRY(cudaEventRecord(e->ev0, e->stream));
     rc = launch_points(e, e->stream, nullptr, nullptr, nullptr, 1, e->h_out_dev, e->d_S, e->d_V);
@@ -657,198 +748,39 @@ int nmch_engine_compute_paths(nmch_engine_t *e, float *S_out, float *V_out, unsi
     return engine_check_guards(e);
 }
 
-// shared by the blocking and the stream form: path kernel (keeps S_T on the device) + strike kernel
-static int strikes_launch(nmch_engine *e, cudaStream_t stream, const float *strikes, int n_strikes, double *d_out4)
-{
-    int rc = ensure_sv(e, (size_t)e->n_local);
-    if (rc) return rc;
-    // reduction slots: 0 = the path kernel's own K = S_0 moments, 1 + 2j / 2 + 2j = strike j
-    const size_t slots = 1 + 2 * (size_t)n_strikes;
-    rc = ensure_buffers(e, slots, (size_t)strike_blocks_per_slot(), (size_t)n_strikes * sizeof(float));
-    if (rc) return rc;
-    CU_TRY(cudaMemcpyAsync(e->d_points, strikes, (size_t)n_strikes * sizeof(float), cudaMemcpyHostToDevice, stream));
-    CU_TRY(cudaStreamSynchronize(stream));                     // `strikes` is caller memory of unknown lifetime
-    rc = launch_points(e, stream, nullptr, nullptr, nullptr, 1, e->h_out_dev, e->d_S, e->d_V);
-    if (rc) return rc;
-    // same stream: the path kernel (and its use of the partial buffer) is complete before the strike kernel starts
-    ReduceBuffers rb{e->d_partials, e->d_tickets + 1, d_out4};
-    CU_TRY(launch_strike_moments(e->d_S, e->n_local, static_cast<const float *>(e->d_points), n_strikes, e->p.S_0, rb, stream));
-    e->launches += 1;
-    return NMCH_OK;
-}
-
 int nmch_engine_compute_strikes(nmch_engine_t *e, const float *strikes, int n_strikes, nmch_strike_moments_t *out)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !out || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    rc = ensure_buffers(e, 1 + 2 * (size_t)n_strikes, 1, 0);   // host-visible result buffer large enough
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = strikes_launch(e, e->stream, strikes, n_strikes, e->h_out_dev + 2);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev1, e->stream));
-    CU_TRY(cudaEventSynchronize(e->ev1));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
-    for (int j = 0; j < n_strikes; ++j) {
-        const double *m = e->h_out + 2 + 4 * (size_t)j;
-        out[j].strike = strikes[j];
-        out[j].sum_payoff = m[0];
-        out[j].sum_payoff_sq = m[1];
-        out[j].sum_delta = m[2];
-        out[j].sum_itm = m[3];
-        out[j].n_paths = e->n_local;
-        out[j].exec_ms = ms;
-    }
-    return engine_check_guards(e);
+    return strike_call(e, strikes, n_strikes, 0, out);
 }
 
 int nmch_engine_compute_strikes_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
                                       double *d_moments)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !d_moments || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    return strikes_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, d_moments);
+    return engine_strike_async(e, cuda_stream, strikes, n_strikes, 0, d_moments);
 }
 
 // ---- strike vector with pathwise delta and vega / sensitivities (FE, native Philox stream) ---------------------------
-// The derivatives of the folded step constants in kappa, theta, sigma and rho (fe_step.cuh), in double, rounded once.
-static TangentFold fold_tangent(const nmch_params_t &p)
-{
-    const double dt = (double)(p.T / (float)p.N);                 // as fold_fe_point forms it
-    const double sdc = std::sqrt(dt) * 1.1774100225154747;         // sqrt(dt) sqrt(2 ln 2)
-    const double rho = (double)p.rho;
-    TangentFold tf;
-    tf.dva_k = (float)(-dt);
-    tf.dvb_k = (float)((double)p.theta * dt);
-    tf.dvb_t = (float)((double)p.k * dt);
-    tf.dvs_s = (float)sdc;
-    tf.dzr_r = (float)sdc;
-    tf.dzc_r = (float)(-rho / std::sqrt(1.0 - rho * rho) * sdc);
-    return tf;
-}
-
-// The native FE pass with the tangent in n_dirs directions (1: compute_greeks, 5: compute_sensitivities), then the fold
-// of 4 + 2 n_dirs raw sums per strike into d_out.
-static int greeks_launch(nmch_engine *e, cudaStream_t stream, const float *strikes, int n_strikes, int n_dirs, double *d_out)
-{
-    const nmch_params_t &p = e->p;
-    const char *what = n_dirs == 1 ? "compute_greeks" : "compute_sensitivities";
-    if (p.method != NMCH_METHOD_FE || p.rng != NMCH_RNG_PHILOX) {
-        char buf[160];
-        std::snprintf(buf, sizeof buf, "%s: the pathwise tangent is carried by the native FE step (method FE, rng PHILOX)", what);
-        return fail(NMCH_ERR_ARG, buf);
-    }
-    if (n_dirs > 1 && !(std::fabs(p.rho) < 1.0f))      // also refuses a NaN rho
-        return fail(NMCH_ERR_ARG, "compute_sensitivities: needs |rho| < 1 (d sqrt(1 - rho^2) / d rho is infinite at |rho| = 1)");
-    int rc = ensure_sv(e, (size_t)e->n_local);
-    if (rc) return rc;
-    const size_t t_need = n_dirs == 1 ? (size_t)e->n_local : (size_t)n_dirs * (size_t)tangent_stride(e->n_local);
-    if (t_need > e->t_cap) {
-        engine_dev_free(e, e->d_T);
-        e->d_T = nullptr;
-        e->t_cap = 0;
-        CU_TRY(engine_dev_malloc(e, (void **)&e->d_T, t_need * sizeof(float), "dS_T/dp"));
-        e->t_cap = t_need;
-    }
-    // reduction slots: 0 = the path kernel's own K = S_0 moments, then 2 + n_dirs per strike (payoff, delta, one per
-    // direction)
-    const size_t slots = 1 + (size_t)(2 + n_dirs) * (size_t)n_strikes;
-    rc = ensure_buffers(e, slots, (size_t)greek_blocks_per_slot(), (size_t)n_strikes * sizeof(float));
-    if (rc) return rc;
-    const unsigned long long tile = (unsigned long long)tangent_tile_paths(n_dirs);
-    const unsigned long long bpp = (e->n_local + tile - 1ull) / tile;
-    if (bpp == 0 || bpp > 0x7fffffffull) return fail(NMCH_ERR_ARG, "launch grid out of range");
-    rc = ensure_buffers(e, 1, (size_t)bpp, 0);
-    if (rc) return rc;
-    CU_TRY(cudaMemcpyAsync(e->d_points, strikes, (size_t)n_strikes * sizeof(float), cudaMemcpyHostToDevice, stream));
-    CU_TRY(cudaStreamSynchronize(stream));                     // `strikes` is caller memory of unknown lifetime
-    FeLaunch L;
-    fill_fe_launch(e, L, 1, (int)bpp, 1);
-    const TangentFold tf = fold_tangent(p);
-    ReduceBuffers rb0{e->d_partials, e->d_tickets, e->h_out_dev};
-    CU_TRY(launch_fe_tangent(L, p.floor, n_dirs, tf, rb0, e->d_S, e->d_V, e->d_T, stream, &e->kinfo));
-    e->draw_offset += 2ull * (unsigned long long)p.N;          // the stream advances like one compute()
-    // same stream: the path kernel (and its use of the partial buffer) is complete before the fold starts
-    ReduceBuffers rb{e->d_partials, e->d_tickets + 1, d_out};
-    CU_TRY(launch_strike_greeks(e->d_S, e->d_T, n_dirs, e->n_local, static_cast<const float *>(e->d_points), n_strikes,
-                                p.S_0, rb, stream));
-    e->launches += 2;
-    return NMCH_OK;
-}
-
 int nmch_engine_compute_greeks(nmch_engine_t *e, const float *strikes, int n_strikes, nmch_greek_moments_t *out)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !out || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    rc = ensure_buffers(e, 1 + 3 * (size_t)n_strikes, 1, 0);   // host-visible result buffer large enough
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = greeks_launch(e, e->stream, strikes, n_strikes, 1, e->h_out_dev + 2);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev1, e->stream));
-    CU_TRY(cudaEventSynchronize(e->ev1));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
-    for (int j = 0; j < n_strikes; ++j) {
-        const double *m = e->h_out + 2 + 6 * (size_t)j;
-        out[j] = nmch_greek_moments_t{strikes[j], m[0], m[1], m[2], m[3], m[4], m[5], e->n_local, ms};
-    }
-    return engine_check_guards(e);
+    return strike_call(e, strikes, n_strikes, 1, out);
 }
 
 int nmch_engine_compute_greeks_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
                                      double *d_moments)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !d_moments || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    return greeks_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, 1, d_moments);
+    return engine_strike_async(e, cuda_stream, strikes, n_strikes, 1, d_moments);
 }
 
 int nmch_engine_compute_sensitivities(nmch_engine_t *e, const float *strikes, int n_strikes,
                                       nmch_sensitivity_moments_t *out)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !out || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    constexpr int kPer = 4 + 2 * NMCH_SENS_COUNT;
-    rc = ensure_buffers(e, 1 + (size_t)(kPer / 2) * (size_t)n_strikes, 1, 0);   // host-visible result buffer large enough
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev0, e->stream));
-    rc = greeks_launch(e, e->stream, strikes, n_strikes, NMCH_SENS_COUNT, e->h_out_dev + 2);
-    if (rc) return rc;
-    CU_TRY(cudaEventRecord(e->ev1, e->stream));
-    CU_TRY(cudaEventSynchronize(e->ev1));
-    float ms = 0.0f;
-    CU_TRY(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
-    for (int j = 0; j < n_strikes; ++j)
-        sensitivity_unpack(e->h_out + 2 + kPer * (size_t)j, strikes[j], e->n_local, ms, &out[j]);
-    return engine_check_guards(e);
+    return strike_call(e, strikes, n_strikes, NMCH_SENS_COUNT, out);
 }
 
 int nmch_engine_compute_sensitivities_async(nmch_engine_t *e, void *cuda_stream, const float *strikes, int n_strikes,
                                             double *d_moments)
 {
-    int rc = check_ready(e);
-    if (rc) return rc;
-    if (!strikes || !d_moments || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceGuard guard(e->device);
-    if (!guard.ok) return fail(NMCH_ERR_CUDA, "cudaSetDevice failed");
-    return greeks_launch(e, static_cast<cudaStream_t>(cuda_stream), strikes, n_strikes, NMCH_SENS_COUNT, d_moments);
+    return engine_strike_async(e, cuda_stream, strikes, n_strikes, NMCH_SENS_COUNT, d_moments);
 }
 
 int nmch_engine_finalize(nmch_engine_t *e)

@@ -63,7 +63,10 @@ int engine_fail(int status, const char *what, cudaError_t err = cudaSuccess);
 cudaError_t engine_dev_malloc(nmch_engine *e, void **ptr, size_t bytes, const char *name);
 void engine_dev_free(nmch_engine *e, void *ptr);
 int engine_check_guards(nmch_engine *e);
-int engine_ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point, size_t point_bytes);
+int engine_ensure_buffers(nmch_engine *e, size_t n_points, size_t blocks_per_point);
+// Copies `bytes` of host records (parameter points, strikes) to e->d_points, growing it as needed, and waits for the copy:
+// the source may be a staging buffer on the caller's stack or caller memory of unknown lifetime.
+int upload_records(nmch_engine *e, cudaStream_t stream, const void *host, size_t bytes);
 
 // em_kernels.cu
 int em_launch_points(nmch_engine *e, cudaStream_t stream, const float *k, const float *theta, const float *sigma,
@@ -80,9 +83,26 @@ void em_release(nmch_engine *e);
 static_assert(NMCH_SENS_COUNT == kNumDirs && NMCH_SENS_V0 == kDirV0 && NMCH_SENS_KAPPA == kDirKappa &&
                   NMCH_SENS_THETA == kDirTheta && NMCH_SENS_SIGMA == kDirSigma && NMCH_SENS_RHO == kDirRho,
               "the header's direction order is the kernels' order");
-// one strike's 14 raw sums (the layout of nmch_engine_compute_sensitivities_async) into the public struct
-inline void sensitivity_unpack(const double *m, float strike, unsigned long long n_paths, float ms,
-                               nmch_sensitivity_moments_t *out)
+// The strike family (compute_strikes, compute_greeks, compute_sensitivities) is one pass with the tangent in n_dirs = 0, 1
+// or NMCH_SENS_COUNT directions.  Per strike it leaves strike_doubles(n_dirs) raw sums: payoff, payoff^2, delta,
+// in-the-money count, then the sum and the sum of squares of 1{S_T > K} dS_T/dp for each direction.
+constexpr int strike_doubles(int n_dirs) { return 4 + 2 * n_dirs; }
+// The stream form of that pass (engine.cu), shared by the engine's and the group's entry points.
+int engine_strike_async(nmch_engine *e, void *cuda_stream, const float *strikes, int n_strikes, int n_dirs, double *d_out);
+
+// one strike's raw sums (strike_doubles(n_dirs) of them, n_dirs as the struct implies) into the public struct
+inline void strike_unpack(const double *m, float strike, unsigned long long n_paths, float ms, nmch_strike_moments_t *out)
+{
+    *out = nmch_strike_moments_t{strike, m[0], m[1], m[2], m[3], n_paths, ms};
+}
+
+inline void strike_unpack(const double *m, float strike, unsigned long long n_paths, float ms, nmch_greek_moments_t *out)
+{
+    *out = nmch_greek_moments_t{strike, m[0], m[1], m[2], m[3], m[4], m[5], n_paths, ms};
+}
+
+inline void strike_unpack(const double *m, float strike, unsigned long long n_paths, float ms,
+                          nmch_sensitivity_moments_t *out)
 {
     out->strike = strike;
     out->sum_payoff = m[0];

@@ -1,16 +1,16 @@
-// greeks_kernels.cu -- strike vector with pathwise delta AND pathwise sensitivities in one pass: the vega d price / d v_0
-// (compute_greeks, ND = 1) or d price / d p for all five of v_0, kappa, theta, sigma, rho (compute_sensitivities, ND = 5)
-// (SURVEY.md §8f rank 2 "a strike vector and pathwise delta/vega reuse the same paths at ~zero RNG cost"; the
-// reference fixes K = S_0 and has no sensitivities, src/NMCH/methods/NMCH.cu:7).
+// greeks_kernels.cu -- the strike family: a strike vector with pathwise delta, and optionally pathwise sensitivities from
+// the same pass: the vega d price / d v_0 (compute_greeks, ND = 1) or d price / d p for all five of v_0, kappa, theta,
+// sigma, rho (compute_sensitivities, ND = 5) (SURVEY.md §8f rank 2 "a strike vector and pathwise delta/vega reuse the
+// same paths at ~zero RNG cost"; the reference fixes K = S_0 and has no sensitivities, src/NMCH/methods/NMCH.cu:7).
 //
 // fe_tangent_kernel<FLOOR, ND>: the native FE step on the native Philox stream (the words, the instructions and therefore
 //   the (S_T, V_T) of fe_philox_kernel, bit for bit) carrying the tangents (dV/dp, dS/dp) of every path in registers;
 //   leaves S_T, V_T and dS_T/dp in HBM (8 + 4 ND bytes per path) and reduces the K = S_0 payoff moments like every path
 //   kernel.
-// strike_greeks_kernel<ND>: folds the terminal arrays per strike: payoff moments, delta = 1{S_T > K} S_T / S_0, and per
+// strike_fold_kernel<ND>: folds the terminal arrays per strike: payoff moments, delta = 1{S_T > K} S_T / S_0, and per
 //   direction 1{S_T > K} dS_T/dp and its square (for the standard error), through the deterministic ticket reduction.
-//   A NaN path makes the strike's payoff, delta and sensitivity sums NaN (DESIGN.md row A3); the in-the-money count stays
-//   a count.
+//   ND = 0 (compute_strikes) folds S_T alone, as left by any path kernel.  A NaN path makes the strike's payoff, delta
+//   and sensitivity sums NaN (DESIGN.md row A3); the in-the-money count stays a count.
 #include "fe_step.cuh"
 #include "kernels.cuh"
 
@@ -126,14 +126,17 @@ fe_tangent_kernel(const __grid_constant__ FeLaunch L, ReduceBuffers rb, float *_
     block_reduce_and_finish(pay, pay2, rb.partials, rb.tickets, rb.out, 0, blockIdx.x, L.blocks_per_point);
 }
 
-constexpr int kGreekThreads = 256;
-constexpr int kGreekBlocks = 296;           // 2 per SM, contiguous slices, 16-byte loads (as strike_moments_kernel)
+constexpr int kFoldThreads = 256;
+constexpr int kFoldBlocks = 296;            // 2 per SM: every block streams a contiguous slice with 16-byte loads
+// per-direction arrays of the fold: ND = 0 keeps one unused element (C++ has no zero-length arrays)
+template <int ND> constexpr int kDirSlots = ND > 0 ? ND : 1;
 
 // One path into the sums of one strike: payoff moments, delta = 1{S_T > K} S_T / S_0, the in-the-money count and, per
 // direction, 1{S_T > K} dS_T/dp and its square.  b[d] is dS_T/dp_d of the path.
 template <int ND>
-__device__ __forceinline__ void greek_fold(float s, const float (&b)[ND], float K, float inv_S0, double &pay, double &pay2,
-                                           double &delta, double &itm, double (&sens)[ND], double (&sens2)[ND])
+__device__ __forceinline__ void greek_fold(float s, const float (&b)[kDirSlots<ND>], float K, float inv_S0, double &pay,
+                                           double &pay2, double &delta, double &itm, double (&sens)[kDirSlots<ND>],
+                                           double (&sens2)[kDirSlots<ND>])
 {
     const double p = payoff_or_nan(s, K);
     pay += p;
@@ -157,17 +160,19 @@ __device__ __forceinline__ void greek_fold(float s, const float (&b)[ND], float 
 }
 
 // Reduction slots of strike j (relative to rb.tickets): (2 + ND) j = (payoff, payoff^2), + 1 = (delta, itm),
-// + 2 + d = (sum, sum of squares) of direction d.  B holds ND arrays of n paths, tangent_stride(n) floats apart.
+// + 2 + d = (sum, sum of squares) of direction d.  B holds ND arrays of n paths, tangent_stride(n) floats apart (not read
+// when ND = 0).
 template <int ND>
-__global__ void __launch_bounds__(kGreekThreads)
-strike_greeks_kernel(const float *__restrict__ S, const float *__restrict__ B, unsigned long long n,
-                     const float *__restrict__ strikes, float inv_S0, ReduceBuffers rb)
+__global__ void __launch_bounds__(kFoldThreads)
+strike_fold_kernel(const float *__restrict__ S, const float *__restrict__ B, unsigned long long n,
+                   const float *__restrict__ strikes, float inv_S0, ReduceBuffers rb)
 {
     constexpr int kSlots = 2 + ND;
     const unsigned long long stride = tangent_stride(n);
     const int j = blockIdx.y;
     const float K = strikes[j];
-    double pay = 0.0, pay2 = 0.0, delta = 0.0, itm = 0.0, sens[ND], sens2[ND];
+    constexpr int NB = kDirSlots<ND>;
+    double pay = 0.0, pay2 = 0.0, delta = 0.0, itm = 0.0, sens[NB], sens2[NB];
 #pragma unroll
     for (int d = 0; d < ND; ++d) sens[d] = sens2[d] = 0.0;
     const unsigned long long n4 = n / 4ull;
@@ -175,23 +180,32 @@ strike_greeks_kernel(const float *__restrict__ S, const float *__restrict__ B, u
     for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
          i += (unsigned long long)gridDim.x * blockDim.x) {
         const float4 s = __ldg(S4 + i);
-        float4 b[ND];
+        if constexpr (ND == 0) {
+            // the loop form of the former S_T-only fold: ptxas schedules it faster than four calls (761 against
+            // 798 us for 64 strikes at 2^24 paths on a B200), with the same additions in the same order
+            const float v[4] = {s.x, s.y, s.z, s.w};
+            const float none[NB] = {};
 #pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            NMCHB_ASSERT(4ull * i + 3ull < stride);
-            b[d] = __ldg(reinterpret_cast<const float4 *>(B + (unsigned long long)d * stride) + i);
+            for (int q = 0; q < 4; ++q) greek_fold<ND>(v[q], none, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
+        } else {
+            float4 b[ND];
+#pragma unroll
+            for (int d = 0; d < ND; ++d) {
+                NMCHB_ASSERT(4ull * i + 3ull < stride);
+                b[d] = __ldg(reinterpret_cast<const float4 *>(B + (unsigned long long)d * stride) + i);
+            }
+            float bx[ND], by[ND], bz[ND], bw[ND];
+#pragma unroll
+            for (int d = 0; d < ND; ++d) { bx[d] = b[d].x; by[d] = b[d].y; bz[d] = b[d].z; bw[d] = b[d].w; }
+            greek_fold<ND>(s.x, bx, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
+            greek_fold<ND>(s.y, by, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
+            greek_fold<ND>(s.z, bz, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
+            greek_fold<ND>(s.w, bw, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
         }
-        float bx[ND], by[ND], bz[ND], bw[ND];
-#pragma unroll
-        for (int d = 0; d < ND; ++d) { bx[d] = b[d].x; by[d] = b[d].y; bz[d] = b[d].z; bw[d] = b[d].w; }
-        greek_fold<ND>(s.x, bx, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
-        greek_fold<ND>(s.y, by, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
-        greek_fold<ND>(s.z, bz, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
-        greek_fold<ND>(s.w, bw, K, inv_S0, pay, pay2, delta, itm, sens, sens2);
     }
     if (blockIdx.x == 0)                                     // ragged tail
         for (unsigned long long i = n4 * 4ull + threadIdx.x; i < n; i += blockDim.x) {
-            float bi[ND];
+            float bi[NB];
 #pragma unroll
             for (int d = 0; d < ND; ++d) {
                 NMCHB_ASSERT(i < n);
@@ -238,20 +252,22 @@ cudaError_t launch_fe_tangent(const FeLaunch &L, int floor_kind, int n_dirs, con
     return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_strike_greeks(const float *d_S, const float *d_B, int n_dirs, unsigned long long n_local,
-                                 const float *d_strikes, int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream)
+cudaError_t launch_strike_fold(const float *d_S, const float *d_B, int n_dirs, unsigned long long n_local,
+                               const float *d_strikes, int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream)
 {
-    dim3 grid(kGreekBlocks, (unsigned)n_strikes, 1);
-    if (n_dirs == 1)
-        strike_greeks_kernel<1><<<grid, kGreekThreads, 0, stream>>>(d_S, d_B, n_local, d_strikes, 1.0f / S0, rb);
+    dim3 grid(kFoldBlocks, (unsigned)n_strikes, 1);
+    if (n_dirs == 0)
+        strike_fold_kernel<0><<<grid, kFoldThreads, 0, stream>>>(d_S, d_B, n_local, d_strikes, 1.0f / S0, rb);
+    else if (n_dirs == 1)
+        strike_fold_kernel<1><<<grid, kFoldThreads, 0, stream>>>(d_S, d_B, n_local, d_strikes, 1.0f / S0, rb);
     else if (n_dirs == kNumDirs)
-        strike_greeks_kernel<kNumDirs><<<grid, kGreekThreads, 0, stream>>>(d_S, d_B, n_local, d_strikes, 1.0f / S0, rb);
+        strike_fold_kernel<kNumDirs><<<grid, kFoldThreads, 0, stream>>>(d_S, d_B, n_local, d_strikes, 1.0f / S0, rb);
     else
         return cudaErrorInvalidValue;
     return cudaGetLastError();
 }
 
-int greek_blocks_per_slot() { return kGreekBlocks; }
+int strike_blocks_per_slot() { return kFoldBlocks; }
 int tangent_tile_paths(int n_dirs)
 {
     return (n_dirs == 1 ? TangentShape<1>::kPaths : TangentShape<kNumDirs>::kPaths) * kTangentThreads;

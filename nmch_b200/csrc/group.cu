@@ -80,70 +80,100 @@ int nccl_fail(const char *what, ncclResult_t r)
     return engine_fail(NMCH_ERR_NCCL, buf);
 }
 
-int ensure_moments(nmch_group *g, size_t n_points)
+int ensure_moments(nmch_group *g, size_t n_doubles)
 {
-    const size_t need = 2 * n_points;
-    if (need <= g->mom_cap) return NMCH_OK;
+    if (n_doubles <= g->mom_cap) return NMCH_OK;
     g->mom_cap = 0;
     for (int i = 0; i < g->n; ++i) {
         GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
         if (g->d_mom[i]) cudaFree(g->d_mom[i]);
         g->d_mom[i] = nullptr;
-        cudaError_t err = cudaMalloc(&g->d_mom[i], need * sizeof(double));
+        cudaError_t err = cudaMalloc(&g->d_mom[i], n_doubles * sizeof(double));
         if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "cudaMalloc(group moments)", err);
     }
     if (g->h_mom) cudaFreeHost(g->h_mom);
     g->h_mom = nullptr;
-    cudaError_t err = cudaMallocHost(&g->h_mom, need * sizeof(double));
+    cudaError_t err = cudaMallocHost(&g->h_mom, n_doubles * sizeof(double));
     if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "cudaMallocHost(group moments)", err);
-    g->mom_cap = need;
+    g->mom_cap = n_doubles;
     return NMCH_OK;
 }
 
-// launches on every device, one grouped allreduce, result of device 0 read back; exec_ms = slowest device
-int run_points(nmch_group *g, const float *k, const float *theta, const float *sigma, int n_points, nmch_moments_t *out)
+// launch_on_device(i) enqueues device i's pass, n_doubles raw sums into g->d_mom[i] on g->stream[i]; then one grouped
+// allreduce, the result of device 0 read back into g->h_mom; *ms = the slowest device's time
+template <class Launch>
+int group_run(nmch_group *g, size_t n_doubles, Launch launch_on_device, float *ms)
 {
-    if (!g || !g->inited) return engine_fail(NMCH_ERR_STATE, "group not initialised");
-    int rc = ensure_moments(g, (size_t)n_points);
+    int rc = ensure_moments(g, n_doubles);
     if (rc) return rc;
     for (int i = 0; i < g->n; ++i) {
         GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
         GROUP_CU_TRY(cudaEventRecord(g->ev0[i], g->stream[i]));
-        rc = k ? nmch_engine_explore_async(g->eng[i], g->stream[i], k, theta, sigma, n_points, g->d_mom[i])
-               : nmch_engine_compute_async(g->eng[i], g->stream[i], g->d_mom[i]);
+        rc = launch_on_device(i);
         if (rc) return rc;
     }
     if (g->n > 1) {
         ncclResult_t r = g_nccl.GroupStart();
         if (r != ncclSuccess) return nccl_fail("ncclGroupStart", r);
         for (int i = 0; i < g->n; ++i) {
-            r = g_nccl.AllReduce(g->d_mom[i], g->d_mom[i], 2 * (size_t)n_points, ncclDouble, ncclSum, g->comm[i], g->stream[i]);
+            r = g_nccl.AllReduce(g->d_mom[i], g->d_mom[i], n_doubles, ncclDouble, ncclSum, g->comm[i], g->stream[i]);
             if (r != ncclSuccess) return nccl_fail("ncclAllReduce", r);
         }
         r = g_nccl.GroupEnd();
         if (r != ncclSuccess) return nccl_fail("ncclGroupEnd", r);
     }
-    float ms = 0.0f;
+    *ms = 0.0f;
     for (int i = 0; i < g->n; ++i) {
         GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
         if (i == 0)
-            GROUP_CU_TRY(cudaMemcpyAsync(g->h_mom, g->d_mom[0], 2 * (size_t)n_points * sizeof(double), cudaMemcpyDeviceToHost, g->stream[0]));
+            GROUP_CU_TRY(cudaMemcpyAsync(g->h_mom, g->d_mom[0], n_doubles * sizeof(double), cudaMemcpyDeviceToHost, g->stream[0]));
         GROUP_CU_TRY(cudaEventRecord(g->ev1[i], g->stream[i]));
     }
     for (int i = 0; i < g->n; ++i) {
         GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
         cudaError_t err = cudaEventSynchronize(g->ev1[i]);
-        if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "group compute", err);
+        if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "group pass", err);
         float t = 0.0f;
         GROUP_CU_TRY(cudaEventElapsedTime(&t, g->ev0[i], g->ev1[i]));
-        if (t > ms) ms = t;
+        if (t > *ms) *ms = t;
     }
+    return NMCH_OK;
+}
+
+// compute (k == nullptr) or explore over n_points on every device
+int run_points(nmch_group *g, const float *k, const float *theta, const float *sigma, int n_points, nmch_moments_t *out)
+{
+    if (!g || !g->inited) return engine_fail(NMCH_ERR_STATE, "group not initialised");
+    float ms = 0.0f;
+    const int rc = group_run(g, 2 * (size_t)n_points, [&](int i) {
+        return k ? nmch_engine_explore_async(g->eng[i], g->stream[i], k, theta, sigma, n_points, g->d_mom[i])
+                 : nmch_engine_compute_async(g->eng[i], g->stream[i], g->d_mom[i]);
+    }, &ms);
+    if (rc) return rc;
     for (int p = 0; p < n_points; ++p) {
         out[p].sum_payoff = g->h_mom[2 * p];
         out[p].sum_payoff_sq = g->h_mom[2 * p + 1];
         out[p].n_paths = g->n_paths;
         out[p].exec_ms = ms;
     }
+    return NMCH_OK;
+}
+
+// the strike family (n_dirs = 0, 1 or NMCH_SENS_COUNT, as the struct T carries) on every device
+template <class T>
+int group_strikes(nmch_group *g, const float *strikes, int n_strikes, int n_dirs, T *out)
+{
+    if (!out) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
+    if (!g || !g->inited) return engine_fail(NMCH_ERR_STATE, "group not initialised");
+    if (!strikes || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
+    DeviceRestore restore;
+    const size_t per = (size_t)nmchb::strike_doubles(n_dirs);
+    float ms = 0.0f;
+    const int rc = group_run(g, per * (size_t)n_strikes, [&](int i) {
+        return nmchb::engine_strike_async(g->eng[i], g->stream[i], strikes, n_strikes, n_dirs, g->d_mom[i]);
+    }, &ms);
+    if (rc) return rc;
+    for (int j = 0; j < n_strikes; ++j) nmchb::strike_unpack(g->h_mom + per * (size_t)j, strikes[j], g->n_paths, ms, &out[j]);
     return NMCH_OK;
 }
 
@@ -209,7 +239,7 @@ static int group_init_impl(nmch_group_t *g, unsigned long long seed)
     }
     g->init_ms = ms;
     g->inited = true;
-    int rc = ensure_moments(g, 1);
+    int rc = ensure_moments(g, 2);
     if (rc == NMCH_OK && g->n > 1) {
         // first collective on a communicator sets up its channels (~100 ms): pay that here, not in compute()
         for (int i = 0; i < g->n; ++i) {
@@ -265,85 +295,19 @@ int nmch_group_explore(nmch_group_t *g, const float *k, const float *theta, cons
     return run_points(g, k, theta, sigma, n_points, out);
 }
 
-// per strike `per` doubles of raw sums: 4 (payoff, payoff^2, delta, itm), 6 (+ vega, vega^2) or 14 (+ five sensitivities
-// and their squares); the last two FE native stream only
-static int group_strikes_impl(nmch_group_t *g, const float *strikes, int n_strikes, int per, float *ms_out)
-{
-    if (!g || !g->inited) return engine_fail(NMCH_ERR_STATE, "group not initialised");
-    if (!strikes || n_strikes <= 0 || n_strikes > NMCH_MAX_STRIKES) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
-    DeviceRestore restore;
-    const size_t count = (size_t)per * (size_t)n_strikes;
-    int rc = ensure_moments(g, (count + 1) / 2);               // ensure_moments counts pairs of doubles
-    if (rc) return rc;
-    for (int i = 0; i < g->n; ++i) {
-        GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
-        GROUP_CU_TRY(cudaEventRecord(g->ev0[i], g->stream[i]));
-        rc = per == 14 ? nmch_engine_compute_sensitivities_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i])
-           : per == 6  ? nmch_engine_compute_greeks_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i])
-                       : nmch_engine_compute_strikes_async(g->eng[i], g->stream[i], strikes, n_strikes, g->d_mom[i]);
-        if (rc) return rc;
-    }
-    if (g->n > 1) {
-        ncclResult_t r = g_nccl.GroupStart();
-        for (int i = 0; i < g->n && r == ncclSuccess; ++i)
-            r = g_nccl.AllReduce(g->d_mom[i], g->d_mom[i], count, ncclDouble, ncclSum, g->comm[i], g->stream[i]);
-        if (r == ncclSuccess) r = g_nccl.GroupEnd();
-        if (r != ncclSuccess) return nccl_fail("strike allreduce", r);
-    }
-    float ms = 0.0f;
-    for (int i = 0; i < g->n; ++i) {
-        GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
-        if (i == 0)
-            GROUP_CU_TRY(cudaMemcpyAsync(g->h_mom, g->d_mom[0], count * sizeof(double), cudaMemcpyDeviceToHost, g->stream[0]));
-        GROUP_CU_TRY(cudaEventRecord(g->ev1[i], g->stream[i]));
-    }
-    for (int i = 0; i < g->n; ++i) {
-        GROUP_CU_TRY(cudaSetDevice(g->dev[i]));
-        cudaError_t err = cudaEventSynchronize(g->ev1[i]);
-        if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "group strikes", err);
-        float t = 0.0f;
-        GROUP_CU_TRY(cudaEventElapsedTime(&t, g->ev0[i], g->ev1[i]));
-        if (t > ms) ms = t;
-    }
-    *ms_out = ms;
-    return NMCH_OK;
-}
-
 int nmch_group_compute_strikes(nmch_group_t *g, const float *strikes, int n_strikes, nmch_strike_moments_t *out)
 {
-    if (!out) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
-    float ms = 0.0f;
-    const int rc = group_strikes_impl(g, strikes, n_strikes, 4, &ms);
-    if (rc) return rc;
-    for (int j = 0; j < n_strikes; ++j) {
-        const double *m = g->h_mom + 4 * (size_t)j;
-        out[j] = nmch_strike_moments_t{strikes[j], m[0], m[1], m[2], m[3], g->n_paths, ms};
-    }
-    return NMCH_OK;
+    return group_strikes(g, strikes, n_strikes, 0, out);
 }
 
 int nmch_group_compute_greeks(nmch_group_t *g, const float *strikes, int n_strikes, nmch_greek_moments_t *out)
 {
-    if (!out) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
-    float ms = 0.0f;
-    const int rc = group_strikes_impl(g, strikes, n_strikes, 6, &ms);
-    if (rc) return rc;
-    for (int j = 0; j < n_strikes; ++j) {
-        const double *m = g->h_mom + 6 * (size_t)j;
-        out[j] = nmch_greek_moments_t{strikes[j], m[0], m[1], m[2], m[3], m[4], m[5], g->n_paths, ms};
-    }
-    return NMCH_OK;
+    return group_strikes(g, strikes, n_strikes, 1, out);
 }
 
 int nmch_group_compute_sensitivities(nmch_group_t *g, const float *strikes, int n_strikes, nmch_sensitivity_moments_t *out)
 {
-    if (!out) return engine_fail(NMCH_ERR_ARG, "bad strike arguments");
-    constexpr int kPer = 4 + 2 * NMCH_SENS_COUNT;
-    float ms = 0.0f;
-    const int rc = group_strikes_impl(g, strikes, n_strikes, kPer, &ms);
-    if (rc) return rc;
-    for (int j = 0; j < n_strikes; ++j) nmchb::sensitivity_unpack(g->h_mom + kPer * (size_t)j, strikes[j], g->n_paths, ms, &out[j]);
-    return NMCH_OK;
+    return group_strikes(g, strikes, n_strikes, NMCH_SENS_COUNT, out);
 }
 
 int nmch_group_finalize(nmch_group_t *g)

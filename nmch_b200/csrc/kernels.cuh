@@ -23,6 +23,7 @@ struct FePoint {
 struct RawPoint {
     float k, theta, sigma, pad;
 };
+static_assert(sizeof(RawPoint) == sizeof(FePoint), "the engine uploads raw records as FePoint{k, theta, sigma, 0}");
 
 struct FeLaunch {
     PhiloxKeys keys;                    // expanded from the seed
@@ -100,19 +101,15 @@ cudaError_t launch_fe_compat(const FeLaunch &L, int floor_kind, const RawPoint *
 cudaError_t launch_fe_xorwow_fast(const FeLaunch &L, int floor_kind, const FePoint *d_pts, XorwowState xs, const uint32_t *skip,
                                   ReduceBuffers rb, float *S_out, float *V_out, cudaStream_t stream, KernelInfo *info);
 
-// strike_kernels.cu: per-strike payoff / delta sums from terminal prices kept on the device
-cudaError_t launch_strike_moments(const float *d_S, unsigned long long n_local, const float *d_strikes, int n_strikes,
-                                  float S0, ReduceBuffers rb, cudaStream_t stream);
-int strike_blocks_per_slot();
-
-// greeks_kernels.cu: native FE pass carrying the pathwise tangent in n_dirs = 1 (v_0) or 5 (v_0, kappa, theta, sigma,
-// rho; fe_step.cuh) directions (leaves S_T, V_T and dS_T/dp of every direction on the device), and the per-strike fold of
-// payoff / delta / sensitivities: 2 + n_dirs reduction slots = 4 + 2 n_dirs doubles per strike
+// greeks_kernels.cu: the native FE pass carrying the pathwise tangent in n_dirs = 1 (v_0) or 5 (v_0, kappa, theta, sigma,
+// rho; fe_step.cuh) directions (leaves S_T, V_T and dS_T/dp of every direction on the device), and the one per-strike
+// fold of every strike-family pass: payoff / delta sums from S_T alone (n_dirs = 0, after any path kernel) or with the
+// sensitivities from d_B as well: 2 + n_dirs reduction slots = 4 + 2 n_dirs doubles per strike
 cudaError_t launch_fe_tangent(const FeLaunch &L, int floor_kind, int n_dirs, const TangentFold &tf, ReduceBuffers rb,
                               float *S_out, float *V_out, float *B_out, cudaStream_t stream, KernelInfo *info);
-cudaError_t launch_strike_greeks(const float *d_S, const float *d_B, int n_dirs, unsigned long long n_local,
-                                 const float *d_strikes, int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream);
-int greek_blocks_per_slot();
+cudaError_t launch_strike_fold(const float *d_S, const float *d_B, int n_dirs, unsigned long long n_local,
+                               const float *d_strikes, int n_strikes, float S0, ReduceBuffers rb, cudaStream_t stream);
+int strike_blocks_per_slot();
 int tangent_tile_paths(int n_dirs);       // paths per block of fe_tangent_kernel
 // floats between the tangent arrays of two directions: n_local rounded up to 16 bytes, so that every array takes float4 loads
 __host__ __device__ inline unsigned long long tangent_stride(unsigned long long n_local) { return (n_local + 3ull) & ~3ull; }

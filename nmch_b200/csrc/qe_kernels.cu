@@ -136,13 +136,12 @@ int qe_launch_points(nmch_engine *e, cudaStream_t stream, const float *k, const 
     std::vector<QePoint> pts(n_points);
     for (int i = 0; i < n_points; ++i)
         pts[i] = own ? fold_qe_point(p, p.k, p.theta, p.sigma) : fold_qe_point(p, k[i], theta[i], sigma[i]);
-    int rc = engine_ensure_buffers(e, n_points, bpp, own ? 0 : (size_t)n_points * sizeof(QePoint));
+    int rc = engine_ensure_buffers(e, n_points, bpp);
     if (rc) return rc;
     const QePoint *d_pts = nullptr;
     if (!own) {
-        cudaError_t err = cudaMemcpyAsync(e->d_points, pts.data(), pts.size() * sizeof(QePoint), cudaMemcpyHostToDevice, stream);
-        if (err == cudaSuccess) err = cudaStreamSynchronize(stream);
-        if (err != cudaSuccess) return engine_fail(NMCH_ERR_CUDA, "QE point upload", err);
+        rc = upload_records(e, stream, pts.data(), pts.size() * sizeof(QePoint));
+        if (rc) return rc;
         d_pts = static_cast<const QePoint *>(e->d_points);
     }
     QeLaunch L{};

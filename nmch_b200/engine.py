@@ -45,6 +45,11 @@ class Moments:
                        self.n_paths + other.n_paths, max(self.exec_ms, other.exec_ms))
 
 
+def _strike_rows(out):
+    """Per strike: payoff moments, pathwise delta and in-the-money share."""
+    return [{"strike": m.strike, "moments": Moments(m.sum_payoff, m.sum_payoff_sq, m.n_paths, m.exec_ms),
+             "delta": m.sum_delta / m.n_paths, "itm": m.sum_itm / m.n_paths} for m in out]
+
 
 def _greek_rows(out):
     """Per strike: payoff moments, pathwise delta, in-the-money share, pathwise vega (d price / d v_0) and its
@@ -76,6 +81,22 @@ def _sensitivity_rows(out):
             row[f"d_{name}_se"] = (var / max(n - 1, 1)) ** 0.5
         rows.append(row)
     return rows
+
+
+def _strike_call(fn, handle, strikes, struct, rows):
+    """One blocking strike-family call of the C ABI (engine or group): fn(handle, strikes, n, out) into an array of
+    `struct`, returned as rows(out)."""
+    strikes = np.ascontiguousarray(strikes, np.float32)
+    out = (struct * len(strikes))()
+    capi.check(fn(handle, strikes.ctypes.data_as(C.POINTER(C.c_float)), len(strikes), out))
+    return rows(out)
+
+
+def _strike_call_async(fn, handle, stream_ptr, strikes, d_moments_ptr):
+    """The stream form of _strike_call: raw sums land in device memory at d_moments_ptr."""
+    strikes = np.ascontiguousarray(strikes, np.float32)
+    capi.check(fn(handle, C.c_void_p(stream_ptr), strikes.ctypes.data_as(C.POINTER(C.c_float)), len(strikes),
+                  C.c_void_p(d_moments_ptr)))
 
 
 class Engine:
@@ -145,54 +166,35 @@ class Engine:
 
     def compute_strikes(self, strikes):
         """One compute() pass priced at a vector of strikes, with the pathwise delta (SURVEY.md §8f rank 2)."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchStrikeMoments * len(strikes))()
-        capi.check(self._lib.nmch_engine_compute_strikes(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                         len(strikes), out))
-        return [{"strike": m.strike, "moments": Moments(m.sum_payoff, m.sum_payoff_sq, m.n_paths, m.exec_ms),
-                 "delta": m.sum_delta / m.n_paths, "itm": m.sum_itm / m.n_paths} for m in out]
+        return _strike_call(self._lib.nmch_engine_compute_strikes, self._h, strikes, capi.NmchStrikeMoments,
+                            _strike_rows)
 
     def compute_strikes_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
         """Enqueue compute_strikes() on a caller stream; raw sums land in device memory (4 doubles per strike:
         payoff, payoff^2, delta, in-the-money count)."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        capi.check(self._lib.nmch_engine_compute_strikes_async(self._h, C.c_void_p(stream_ptr),
-                                                               strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                               len(strikes), C.c_void_p(d_moments_ptr)))
+        _strike_call_async(self._lib.nmch_engine_compute_strikes_async, self._h, stream_ptr, strikes, d_moments_ptr)
 
     def compute_greeks(self, strikes):
         """compute_strikes() plus the pathwise vega d E[(S_T - K)^+] / d v_0 (FE, native Philox stream only)."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchGreekMoments * len(strikes))()
-        capi.check(self._lib.nmch_engine_compute_greeks(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                        len(strikes), out))
-        return _greek_rows(out)
+        return _strike_call(self._lib.nmch_engine_compute_greeks, self._h, strikes, capi.NmchGreekMoments, _greek_rows)
 
     def compute_greeks_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
         """Enqueue compute_greeks() on a caller stream; raw sums land in device memory (6 doubles per strike:
         payoff, payoff^2, delta, in-the-money count, vega, vega^2)."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        capi.check(self._lib.nmch_engine_compute_greeks_async(self._h, C.c_void_p(stream_ptr),
-                                                              strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                              len(strikes), C.c_void_p(d_moments_ptr)))
+        _strike_call_async(self._lib.nmch_engine_compute_greeks_async, self._h, stream_ptr, strikes, d_moments_ptr)
 
     def compute_sensitivities(self, strikes):
         """compute_strikes() plus the pathwise sensitivities of E[(S_T - K)^+] to v_0, kappa, theta, sigma and rho from
         the same pass (FE, native Philox stream only; |rho| < 1).  Rows carry "d_v0", "d_kappa", "d_theta", "d_sigma",
         "d_rho" and their standard errors "d_<p>_se"."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchSensitivityMoments * len(strikes))()
-        capi.check(self._lib.nmch_engine_compute_sensitivities(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                               len(strikes), out))
-        return _sensitivity_rows(out)
+        return _strike_call(self._lib.nmch_engine_compute_sensitivities, self._h, strikes, capi.NmchSensitivityMoments,
+                            _sensitivity_rows)
 
     def compute_sensitivities_async(self, stream_ptr: int, strikes, d_moments_ptr: int) -> None:
         """Enqueue compute_sensitivities() on a caller stream; raw sums land in device memory (14 doubles per strike:
         payoff, payoff^2, delta, in-the-money count, then sum and sum of squares for v_0, kappa, theta, sigma, rho)."""
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        capi.check(self._lib.nmch_engine_compute_sensitivities_async(self._h, C.c_void_p(stream_ptr),
-                                                                     strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                                     len(strikes), C.c_void_p(d_moments_ptr)))
+        _strike_call_async(self._lib.nmch_engine_compute_sensitivities_async, self._h, stream_ptr, strikes,
+                           d_moments_ptr)
 
     def check(self) -> None:
         """Synchronise and, in the checked build, sweep the guard bands / surface a failed device assert."""
@@ -267,26 +269,14 @@ class Group:
         return [Moments(m.sum_payoff, m.sum_payoff_sq, m.n_paths, m.exec_ms) for m in out]
 
     def compute_strikes(self, strikes):
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchStrikeMoments * len(strikes))()
-        capi.check(self._lib.nmch_group_compute_strikes(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                        len(strikes), out))
-        return [{"strike": m.strike, "moments": Moments(m.sum_payoff, m.sum_payoff_sq, m.n_paths, m.exec_ms),
-                 "delta": m.sum_delta / m.n_paths, "itm": m.sum_itm / m.n_paths} for m in out]
+        return _strike_call(self._lib.nmch_group_compute_strikes, self._h, strikes, capi.NmchStrikeMoments, _strike_rows)
 
     def compute_greeks(self, strikes):
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchGreekMoments * len(strikes))()
-        capi.check(self._lib.nmch_group_compute_greeks(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                       len(strikes), out))
-        return _greek_rows(out)
+        return _strike_call(self._lib.nmch_group_compute_greeks, self._h, strikes, capi.NmchGreekMoments, _greek_rows)
 
     def compute_sensitivities(self, strikes):
-        strikes = np.ascontiguousarray(strikes, np.float32)
-        out = (capi.NmchSensitivityMoments * len(strikes))()
-        capi.check(self._lib.nmch_group_compute_sensitivities(self._h, strikes.ctypes.data_as(C.POINTER(C.c_float)),
-                                                              len(strikes), out))
-        return _sensitivity_rows(out)
+        return _strike_call(self._lib.nmch_group_compute_sensitivities, self._h, strikes, capi.NmchSensitivityMoments,
+                            _sensitivity_rows)
 
     @property
     def size(self) -> int:

@@ -97,7 +97,7 @@ def kernel_split(e, strikes, reps):
         if ev.device_type.name != "CUDA" or ev.count == 0:
             continue
         name = ev.key
-        tag = "tangent_kernel" if "fe_tangent_kernel" in name else "fold" if "strike_greeks_kernel" in name else None
+        tag = "tangent_kernel" if "fe_tangent_kernel" in name else "fold" if "strike_fold_kernel" in name else None
         if tag:
             t = getattr(ev, "device_time_total", None)
             if t is None:
