@@ -842,7 +842,8 @@ void orc_qe_run(const orc_params_t *p, uint64_t seed, uint64_t first_path, uint6
                 c2 = (float)(theta * sigma * sigma * om * om / (2.0 * k));
     const double dK2 = 0.5 * dt * (k * rho / sigma - 0.5) + rho / sigma, dK3 = 0.5 * dt * (1.0 - rho * rho);
     const float K2 = (float)dK2, K3 = (float)dK3, K4 = (float)dK3, A = (float)(dK2 + 0.5 * dK3);
-    const float r_dt = p->r * (p->T / (float)p->N), lnS0 = (float)log((double)p->S_0), K = p->S_0;
+    const float hV = (float)(-0.5 * (dK3 + dK3 * e)), h0 = (float)((double)(p->r * (p->T / (float)p->N)) - 0.5 * dK3 * theta * om);
+    const float K = p->S_0;
     const uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
     double acc = 0.0, acc2 = 0.0;
     if (threads <= 0) threads = orc_max_threads();
@@ -851,7 +852,7 @@ void orc_qe_run(const orc_params_t *p, uint64_t seed, uint64_t first_path, uint6
 #endif
     for (int64_t i = 0; i < (int64_t)n_paths; ++i) {
         const uint64_t g = first_path + (uint64_t)i;
-        float V = p->v_0, lnS = lnS0;
+        float V = p->v_0, lnS = 0.0f;     /* ln(S / S_0), as the kernel accumulates it */
         for (int n = 0; n < p->N; ++n) {
             const uint32_t ctr[4] = {(uint32_t)n, call, (uint32_t)g, (uint32_t)(g >> 32)};
             uint32_t w[4];
@@ -861,22 +862,31 @@ void orc_qe_run(const orc_params_t *p, uint64_t seed, uint64_t first_path, uint6
             const float ang = (1.0f + (float)(w[1] >> 9) * 1.1920929e-07f) * 6.2831855f;
             const float zv = rad * sinf(ang), zs = rad * cosf(ang);
             const float u = ((float)(w[2] >> 9) + 0.5f) * 1.1920929e-07f;
-            const float m = fmaf(V, fe, m0), s2 = fmaf(V, c1, c2), psi = s2 / (m * m);
-            float Vn, lnM;
+            const float m = fmaf(V, fe, m0), s2 = fmaf(V, c1, c2), mm = m * m, psi = s2 / mm;
+            /* dlog = K2 (V' - m) - (ln M - A m): the kernel's form of K2 V' - ln M without the cancellation */
+            float Vn, dlog;
             if (psi <= 1.5f) {
                 const float t = 2.0f / psi, b2 = t - 1.0f + sqrtf(t * (t - 1.0f)), a = m / (1.0f + b2);
-                const float q = sqrtf(b2) + zv, den = fmaxf(1.0f - 2.0f * A * a, 1e-6f);
+                const float b = sqrtf(b2), q = b + zv, dV = a * fmaf(zv, fmaf(2.0f, b, zv), -1.0f);
+                const float x = 2.0f * A * a, den = fmaxf(1.0f - x, 1e-6f);
                 Vn = a * q * q;
-                lnM = A * b2 * a / den - 0.5f * logf(den);
+                const float tail = fabsf(x) < 0.0625f ? x * x * fmaf(x, fmaf(x, fmaf(x, 0.2f, 0.25f), 0.33333334f), 0.5f)
+                                                      : -(logf(den) + x);
+                dlog = fmaf(K2, dV, 0.5f * fmaf(b2 * x, -x / den, -tail));
             } else {
                 const float pp = (psi - 1.0f) / (psi + 1.0f), beta = (1.0f - pp) / m;
                 Vn = (u <= pp) ? 0.0f : logf((1.0f - pp) / (1.0f - u)) / beta;
-                lnM = logf(pp + beta * (1.0f - pp) / fmaxf(beta - A, 1e-6f));
+                const float lnM = logf(pp + beta * (1.0f - pp) / fmaxf(beta - A, 1e-6f));
+                dlog = fmaf(K2, Vn - m, fmaf(A, m, -lnM));
             }
-            lnS += r_dt - lnM - 0.5f * K3 * V + K2 * Vn + sqrtf(fmaf(K3, V, K4 * Vn)) * zs;
+            if (!(mm >= 1.17549435e-38f)) {     /* absorbed at zero: theta = 0 and V = 0, or m^2 below FLT_MIN */
+                Vn = 0.0f;
+                dlog = 0.0f;
+            }
+            lnS += fmaf(hV, V, h0) + dlog + sqrtf(fmaf(K3, V, K4 * Vn)) * zs;
             V = Vn;
         }
-        const float S = expf(lnS), pay = fmaxf(0.0f, S - K);
+        const float S = p->S_0 * expf(lnS), pay = fmaxf(0.0f, S - K);
         acc += (double)pay;
         acc2 += (double)pay * (double)pay;
         if (S_out) S_out[i] = S;

@@ -57,9 +57,9 @@ def test_em_random_configurations_track_oracle(rng):
 
 def test_qe_random_configurations_match_restatement():
     from nmch_b200 import engine as E
+    # every rho of the box, up to 0.5: the martingale correction exists there (1 - 2 A a > 0 and beta > A for V in
+    # [0, 2]; test_qe64_reference.test_martingale_correction_exists_in_the_fuzz_box_with_positive_rho)
     for c in _configs(3000, 10):
-        if c["rho"] > 0.2:
-            continue                                        # QE's martingale correction needs A < 1/(2a): keep rho <= 0.2
         kw = {k: c[k] for k in ("T", "S_0", "v_0", "r", "k", "rho", "theta", "sigma")}
         with E.Engine(NTPB=1, NB=1, N=c["N"], method=E.METHOD_QE, n_paths=c["first"] + c["n"], first_path=c["first"],
                       n_local=c["n"], **kw) as e:
